@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the MicrobeCensus hot path on B200: reads/s end-to-end AGS (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c4] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--workload c3|c2|c4] [--impl ours|reference] [--dump-outputs DIR]
 
 One step = one pass of the whole hot path over one batch of synthetic reads: read QC -> 6-frame
 translation + SEG + seeding + ungapped X-drop -> gapped X-drop -> per-read classification -> per-family
@@ -18,6 +18,10 @@ processes paired files one after the other); c2 = 2,000,000 synthetic 100 bp sin
 `roofline` = the seed+ungapped kernel against measured HBM bandwidth (algorithmic bytes, DESIGN.md section 5);
 `cpu_baseline` = the unmodified reference (baseline/_ref: its Python stages + rapsearch_Linux_2.15 -z <cores>)
 on a bounded prefix of the same reads, or the CPU oracle port when the reference install is absent.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last step of each arm computed (device_*.npy, e2e_*.npy:
+ags, agg_hits in family order, counts = SearchResult.counts_vector(), classified = best subject per read, hits = the
+HSPs), so that two builds can be compared output for output on the same seeded reads.
 """
 import argparse
 import json
@@ -57,7 +61,44 @@ def parse():
     p.add_argument("--reads-per-gpu", type=int, default=None)
     p.add_argument("--ref-sample", type=int, default=20000, help="reads per step of the CPU reference arm")
     p.add_argument("--no-cpu-baseline", action="store_true")
-    return p.parse_args()
+    p.add_argument("--dump-outputs", metavar="DIR", default=None,
+                   help="write what the last timed step of each arm computed to DIR/<name>.npy (float64)")
+    a = p.parse_args()
+    if a.steps < 1:
+        p.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        p.error("--dump-outputs records the GPU arm (--impl ours)")
+    return a
+
+
+# caps of the per-read and per-HSP arrays in a dump: 2 arms x (500k + 160k x 12) float64 values = 39 MB at most
+DUMP_READS, DUMP_HITS, DUMP_SEED = 500_000, 160_000, 20260105
+
+
+def outputs_of_step(eng, markers, ags, res, n_reads):
+    """What a caller of one step receives (AGS, per-family sums, the counters) plus the per-read classification and
+    the HSPs the step left in the context, as float64 arrays.  Reads and HSPs beyond the caps are a fixed, seeded
+    sample of rows (the same rows for the same counts)."""
+    import numpy as np
+
+    def sample(a, cap):
+        if len(a) <= cap:
+            return a
+        return a[np.sort(np.random.default_rng(DUMP_SEED).choice(len(a), cap, replace=False))]
+    agg = res.agg_hits()
+    return {"ags": np.array([ags], np.float64),
+            "agg_hits": np.array([agg.get(f, 0.0) for f in markers.fam_names], np.float64),
+            "counts": res.counts_vector().astype(np.float64),
+            "classified": sample(eng.classified(n_reads), DUMP_READS).astype(np.float64),
+            "hits": sample(eng.hits(), DUMP_HITS).astype(np.float64)}
+
+
+def write_outputs(path, arms):
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for arm, arrays in arms.items():
+        for name, arr in arrays.items():
+            np.save(os.path.join(path, "%s_%s.npy" % (arm, name)), arr)
 
 
 # ---------------------------------------------------------------------------------------------- clocks
@@ -406,7 +447,11 @@ def main():
         sampler.start()
     ms_dev, wall_dev, stage_dev, launches, (ags, res) = timed(step_device, a.steps, max(a.warmup, 3))
     clocks = sampler.stop() if sampler else None
+    dump = {"device": outputs_of_step(eng, markers, ags, res, n)} if a.dump_outputs and rank == 0 else None
     ms_e2e, wall_e2e, stage_e2e, _, (ags2, res2) = timed(step_e2e, a.steps, 1)
+    if dump is not None:
+        dump["e2e"] = outputs_of_step(eng, markers, ags2, res2, n)
+        write_outputs(a.dump_outputs, dump)
     # device events bracket only GPU work; the step also holds host work (counter read-back, AGS estimate),
     # so the step time is the larger of the two clocks
     t_dev = max(ms_dev / 1e3, wall_dev)

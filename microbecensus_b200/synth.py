@@ -21,7 +21,7 @@ _genome = None
 
 def genome_pack_path():
     """data/genomes30.pack (all 30 training genomes of the reference, 84.8 Mbp, SURVEY 8d; written by
-    tools/build_genome_pack.py --all at build time where the reference tree is mounted) if present, else the committed
+    `tools/build_genome_pack.py --all` from a reference checkout, kept out of git) if present, else the committed
     ten-genome data/genomes.pack; $MCX_GENOME_PACK overrides."""
     if os.environ.get("MCX_GENOME_PACK"):
         return os.environ["MCX_GENOME_PACK"]

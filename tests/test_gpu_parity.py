@@ -472,3 +472,31 @@ def test_m8_dump_matches_rapsearch_lines(eng, markers, tmp_path):
     single = [l for l in ref if len(l.split("\t")[10].split(".")[-1]) <= 2]
     same = sum(l in ours for l in single)
     assert same >= 0.99 * len(single), (same, len(single))
+
+
+def test_bench_dump_outputs_are_the_last_step(eng, markers, tmp_path):
+    """bench.py --dump-outputs: what the last timed step of both arms computed (AGS, per-family sums, counters, the
+    classification of every read, the HSPs) as float64 .npy files, equal to one search of the same seeded reads."""
+    import json, subprocess, sys
+    root = os.path.dirname(os.path.dirname(golden_io.GOLD))
+    n = 20000
+    out = tmp_path / "dump"
+    cp = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--workload", "c2", "--reads-per-gpu", str(n), "--steps", "2",
+                         "--warmup", "0", "--no-cpu-baseline", "--dump-outputs", str(out)], capture_output=True, text=True, cwd=str(tmp_path))
+    assert cp.returncode == 0, cp.stderr[-2000:]
+    assert json.loads(cp.stdout.strip().splitlines()[-1])["steps"] == 2
+    got = {p.stem: np.load(p) for p in out.glob("*.npy")}
+    assert set(got) == {"%s_%s" % (arm, k) for arm in ("device", "e2e") for k in ("ags", "agg_hits", "counts", "classified", "hits")}
+    assert all(a.dtype == np.float64 for a in got.values()) and sum(a.nbytes for a in got.values()) <= 64 << 20
+    eng.set_params(100)
+    eng.push(synth.reads(2, 0, n, 100))
+    res = eng.search(-1)
+    agg = res.agg_hits()
+    ags = mcb.estimate_average_genome_size({"read_length": 100, "sampled_reads": n, "verbose": False}, None, agg)
+    assert res.sampled_reads == n and len(got["device_hits"]) > 1000
+    for arm in ("device", "e2e"):
+        assert got[arm + "_ags"].tolist() == [ags]
+        assert got[arm + "_agg_hits"].tolist() == [agg.get(f, 0.0) for f in markers.fam_names]
+        assert np.array_equal(got[arm + "_counts"], res.counts_vector())
+        assert np.array_equal(got[arm + "_classified"], eng.classified(n))
+        assert np.array_equal(got[arm + "_hits"], eng.hits())

@@ -14,7 +14,6 @@ from microbecensus_b200 import _lib, microbe_census as mcb
 from microbecensus_b200.engine import ReadBatch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 def test_abi_library_exports_every_declared_symbol():
@@ -114,25 +113,29 @@ def test_reader_matches_readfq_state_machine(tmp_path):
                 assert b.quals[b.offsets[i]:b.offsets[i + 1]].tobytes().decode() == r.quality[:len(r.seq)], name
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted")
 def test_reader_and_autodetect_match_reference_on_its_own_files():
-    sys.path.insert(0, os.path.join(ROOT, "baseline", "_ref"))
-    import warnings
-    warnings.filterwarnings("ignore")
-    from microbe_census import microbe_census as ref
-    for path, ft in ((os.path.join(REF, "microbe_census/example/example.fq.gz"), "fastq"),
-                     (os.path.join(REF, "microbe_census/example/example.fa.gz"), "fasta")):
-        recs = list(ref.parse_seqs(ref.open_file(path)))
+    """The reference's example and test inputs (copies in tests/golden/full): records, total bases, detected file type,
+    read length and quality offset, and count_bases as the unmodified reference reported them (full/expected.json)."""
+    exp = golden_io.read_json(os.path.join("full", "expected.json"))
+    for key in ("example_fq", "example_fa_500", "metagenome"):
+        e = exp[key]
+        name = os.path.join("full", e["file"])
+        path = os.path.join(golden_io.GOLD, name)
+        ft = "fasta" if e["quality_offset"] is None else "fastq"     # the reference detects a quality offset for FASTQ only
+        seqs = [r[1] for r in golden_io.read_fastq(name)] if ft == "fastq" else golden_io.read_fasta(name)
         b = mcb.load_reads(path, ft)
-        assert b.n == len(recs)
-        assert int(b.offsets[-1]) == sum(len(r.seq) for r in recs)
-        for i in range(0, len(recs), 97):
-            assert b.bases[b.offsets[i]:b.offsets[i + 1]].tobytes().decode() == recs[i].seq
-        assert mcb.auto_detect_file_type(path) == ref.auto_detect_file_type(path)
-        assert mcb.auto_detect_read_length(path, ft) == ref.auto_detect_read_length(path, ft)
-    fq = os.path.join(REF, "microbe_census/example/example.fq.gz")
-    assert mcb.auto_detect_quality_offset(fq) == ref.auto_detect_quality_offset(fq)
-    assert mcb.count_bases({"seqfiles": [fq], "verbose": False, "file_type": "fastq"}) == ref.count_bases({"seqfiles": [fq], "verbose": False})
+        assert b.n == len(seqs)
+        assert int(b.offsets[-1]) == sum(len(s) for s in seqs) == e["total_bases"]
+        for i in range(0, len(seqs), 97):
+            assert b.bases[b.offsets[i]:b.offsets[i + 1]].tobytes().decode() == seqs[i]
+        assert mcb.auto_detect_file_type(path) == ft
+        if "read_length" not in e["opts"]:          # detected by the reference
+            assert mcb.auto_detect_read_length(path, ft) == e["read_length"]
+        else:                                       # 500 bp reads only: the longest length the reference supports
+            assert mcb.auto_detect_read_length(path, ft) == 500
+        if ft == "fastq":
+            assert mcb.auto_detect_quality_offset(path) == e["quality_offset"]
+        assert mcb.count_bases({"seqfiles": [path], "verbose": False, "file_type": ft}) == e["total_bases"]
 
 
 def test_oracle_qc_matches_reference_counters(oracle):

@@ -1,13 +1,13 @@
 """libmcxio (C++ FASTA/FASTQ reader, include/mcxio.h) against the readfq generator it restates
-(mc.py:294-325, mirrored by microbecensus_b200.microbe_census.parse_seqs) and, when the reference tree is
-mounted, against the reference's own parse_seqs / count_bases.  No GPU needed."""
+(mc.py:294-325, mirrored by microbecensus_b200.microbe_census.parse_seqs) and against what the reference's own
+parse_seqs / count_bases returned (tests/golden).  No GPU needed."""
 import bz2
 import gzip
 import io
+import json
 import os
 import random
 import re
-import sys
 
 import numpy as np
 import pytest
@@ -15,7 +15,7 @@ import pytest
 from microbecensus_b200 import microbe_census as mcb, seqio
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+GOLD = os.path.join(ROOT, "tests", "golden")
 
 CASES = {
     "multi-line fasta, names with spaces, no final newline": ">r1 desc\nACGT\nAC\n>r2\nTTTT\n>r3\n\nGG",
@@ -227,17 +227,17 @@ def test_corrupt_gzip_is_an_error(tmp_path):
             f.next_batch()
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="reference tree not mounted")
 def test_against_the_reference_generator():
-    sys.path.insert(0, os.path.join(ROOT, "baseline", "_ref"))
-    import warnings
-    warnings.filterwarnings("ignore")
-    from microbe_census import microbe_census as ref
+    """The records of the reference's own generator on every shape (tests/golden/readfq_cases.json), and its count_bases
+    on its example and test inputs (copies and totals in tests/golden/full)."""
+    gold = json.load(open(os.path.join(GOLD, "readfq_cases.json")))["cases"]
+    assert set(gold) == set(CASES)
     for label, text in CASES.items():
-        want = [(r.seq, r.quality) for r in ref.parse_seqs(io.StringIO(text, newline=None))]
+        assert gold[label]["text"] == text, label
+        want = [(s, q) for s, q in gold[label]["records"]]
         check(seqio.SeqFile.from_bytes(text.encode()).next_batch(), want, label)
-    for rel in ("microbe_census/example/example.fq.gz", "microbe_census/example/example.fa.gz", "tests/data/metagenome.fa.gz"):
-        path = os.path.join(REF, rel)
-        with seqio.SeqFile(path) as f:
+    exp = json.load(open(os.path.join(GOLD, "full", "expected.json")))
+    for key in ("example_fq", "example_fa_500", "metagenome"):
+        with seqio.SeqFile(os.path.join(GOLD, "full", exp[key]["file"])) as f:
             n, total = f.skip_rest()
-        assert total == ref.count_bases({"seqfiles": [path], "verbose": False}), rel
+        assert total == exp[key]["total_bases"], key
