@@ -2290,6 +2290,64 @@ __global__ void k_keep_sorted(const uint8_t *__restrict__ keep, int64_t n, int32
 // host side
 // ------------------------------------------------------------------------------------------------
 constexpr int MAX_COPY_STEPS = 64;             // host->device copies of a push are cut into at most this many steps
+struct mcx_ctx;
+static int fail(mcx_ctx *ctx, int code, const std::string &msg);
+#define CK(call)                                                                                   \
+    do {                                                                                           \
+        cudaError_t e_ = (call);                                                                   \
+        if (e_ != cudaSuccess)                                                                     \
+            return fail(ctx, MCX_ECUDA, std::string(#call) + ": " + cudaGetErrorString(e_));       \
+    } while (0)
+#define TRY(call)                                                                                  \
+    do { const int rc_ = (call); if (rc_ != MCX_OK) return rc_; } while (0)
+
+template <typename T>
+static cudaError_t dev_alloc(T **p, size_t n) { return cudaMalloc((void **)p, n * sizeof(T) ? n * sizeof(T) : 1); }
+
+// a device buffer with its capacity in entries; a borrowed one (caller's storage, mcx_push_reads*_dev) has capacity 0,
+// is never freed here, and the next ensure() replaces it with storage of the context's own
+template <typename T>
+struct DevBuf {
+    T *p = nullptr;
+    int64_t cap = 0;
+    bool owned = true;
+    DevBuf() = default;
+    DevBuf(const DevBuf &) = delete;
+    DevBuf &operator=(const DevBuf &) = delete;
+    ~DevBuf() { if (owned && p) cudaFree(p); }
+    operator T *() const { return p; }
+    int release(mcx_ctx *ctx) {
+        if (owned && p) CK(cudaFree(p));
+        p = nullptr; cap = 0; owned = true;
+        return MCX_OK;
+    }
+    // room for `need` entries, contents not kept: free, then allocate need + need/8 + slack; *grew: it reallocated
+    int ensure(mcx_ctx *ctx, int64_t need, bool *grew = nullptr, int64_t slack = 16) {
+        if (grew) *grew = false;
+        if (cap >= need && p) return MCX_OK;
+        TRY(release(ctx));
+        CK(dev_alloc(&p, (size_t)(need + need / 8 + slack)));
+        cap = need + need / 8 + slack;
+        if (grew) *grew = true;
+        return MCX_OK;
+    }
+    // exactly `cap` entries, the first `keep` copied over (on the context's stream, waited for before the old one is freed)
+    int grow_keep(mcx_ctx *ctx, int64_t keep, int64_t cap);
+    int borrow(mcx_ctx *ctx, T *q) {
+        TRY(release(ctx));
+        p = q; owned = false;
+        return MCX_OK;
+    }
+};
+
+// events of the context's streams, named by the point they mark (0: start of a span, 1: end)
+enum Ev { EV_QC0, EV_QC1, EV_KQC0, EV_KQC1, EV_DEDUP0, EV_DEDUP1, EV_H2D0, EV_LENS, EV_H2D1, EV_FRAMES0, EV_SEG0, EV_PROBE0, EV_KPROBE1,
+          EV_SEED0, EV_KSEED1, EV_GAP0, EV_GAP1, EV_SORT0, EV_CLS0, EV_D2H0, EV_D2H1, EV_BENCH0, EV_BENCH1 /* microbenchmarks */, EV_N };
+// slots of mcx_timings (include/mcx.h) and of mcx_timings_detail
+enum Ms { MS_H2D, MS_QC, MS_PROBE, MS_GAPPED, MS_SORT, MS_CLASSIFY, MS_D2H, MS_EXTEND, MS_FRAMES, MS_SEG, MS_KQC, MS_DEDUP, MS_N };
+enum MsDetail { MSD_KPROBE, MSD_KRESOLVE, MSD_KSEED, MSD_KWALK, MSD_N };
+static_assert(MS_N == 12 && MSD_N == 4, "mcx_timings fills 12 slots, mcx_timings_detail 4");
+
 struct mcx_ctx {
     int device = 0;
     cudaStream_t stream = nullptr;             // kernels
@@ -2301,83 +2359,70 @@ struct mcx_ctx {
     // database
     DevDB db{};
     std::vector<void *> db_allocs;
-    int n_subj = 0;
     // read store (see ReadStore)
     int64_t n_reads = 0, n_words = 0, n_bases = 0;
-    uint32_t *d_pk = nullptr, *d_len = nullptr;
-    int64_t *d_woff = nullptr, *d_qoff = nullptr;
-    uint8_t *d_quals = nullptr;
+    DevBuf<uint32_t> d_pk, d_len;
+    DevBuf<int64_t> d_woff, d_qoff;
+    DevBuf<uint8_t> d_quals;
     bool have_quals = false;
-    bool ext_pk = false, ext_len = false, ext_quals = false;   // buffers owned by the caller (mcx_push_reads*_dev)
-    int64_t cap_pk = 0, cap_len = 0, cap_woff = 0, cap_qoff = 0, cap_quals = 0;
     // ASCII staging of mcx_push_reads / mcx_push_reads_dev
-    uint8_t *d_ascii = nullptr;
-    int64_t *d_aoffs = nullptr;
-    int64_t cap_ascii = 0, cap_aoffs = 0;
+    DevBuf<uint8_t> d_ascii;
+    DevBuf<int64_t> d_aoffs;
     // progress of the host -> device copies: step k covers packed words [k * step_words, ...) and quality bytes
     // [k * step_qbytes, ...); ev_copy[k] is recorded behind it on the copy stream
     int n_steps = 0;                           // 0: nothing to wait for (device-resident push, or everything already waited on)
     int steps_waited = 0;
     int64_t step_words = 0, step_qbytes = 0;
-    cudaEvent_t ev_copy[MAX_COPY_STEPS] = {nullptr}, ev_len = nullptr, ev_h2d0 = nullptr;
+    cudaEvent_t ev_copy[MAX_COPY_STEPS] = {nullptr};
     // QC state
-    uint8_t *d_code = nullptr;
-    FpKey *d_fp = nullptr;
-    unsigned long long *d_fpa = nullptr, *d_fpa2 = nullptr;
-    uint32_t *d_fpi = nullptr, *d_fpi2 = nullptr;
-    int64_t cap_fp = 0, cap_fpa = 0, cap_fpa2 = 0, cap_fpi = 0, cap_fpi2 = 0;
-    int32_t *d_kept = nullptr;
-    int64_t cap_code = 0, cap_kept = 0;
+    DevBuf<uint8_t> d_code;
+    DevBuf<FpKey> d_fp;
+    DevBuf<unsigned long long> d_fpa, d_fpa2;
+    DevBuf<uint32_t> d_fpi, d_fpi2;
+    DevBuf<int32_t> d_kept;
     // fingerprints of the reads kept by earlier pushes of the run (streamed -d)
-    unsigned long long *d_store_a = nullptr, *d_store_b = nullptr;
-    int64_t cap_store = 0, n_store = 0;
+    DevBuf<unsigned long long> d_store_a, d_store_b;
+    int64_t n_store = 0;
     // cross-GPU -d exchange
-    long long *d_xsend = nullptr;
-    uint8_t *d_xmarks = nullptr;
-    unsigned long long *d_xkg = nullptr;
-    uint32_t *d_xvi = nullptr;
-    int64_t cap_xsend = 0, cap_xmarks = 0, cap_xkg = 0, cap_xvi = 0, x_nsend = 0;
+    DevBuf<long long> d_xsend;
+    DevBuf<uint8_t> d_xmarks;
+    DevBuf<unsigned long long> d_xkg;
+    DevBuf<uint32_t> d_xvi;
+    int64_t x_nsend = 0;
     int64_t qc_upto = 0;                       // reads [0, qc_upto) have their verdict
     bool dedup_done = false, fp_done = false, counts_valid = false, kqc_pending = false;
     bool h2d_timed = false;                    // the last push recorded its copy events (host pushes only)
     mcx_qc qc{};
     bool pushed = false, searched = false;
     // search buffers
-    uint4 *d_surv = nullptr;
-    uint8_t *d_frames = nullptr;
-    uint32_t *d_segq = nullptr, *d_segm = nullptr;
-    unsigned long long *d_seen = nullptr;     // k_walk's duplicate filter
-    uint4 *d_seedq = nullptr;                 // accepted seeds between k_seed and k_walk
-    int64_t cap_seen = 0, cap_seedq = 0;
-    unsigned long long *d_gitems = nullptr;   // gapped work lists: three regions of 2 * survivors entries
-    GExtRec *d_gext = nullptr;
-    uint32_t *d_dirs = nullptr;               // direction nibbles of k_gap_dp for k_gap_trace
-    int64_t cap_gitems = 0, cap_gext = 0, cap_dirs = 0;
-    int64_t cap_segq = 0, cap_segm = 0;
-    Cand *d_cand = nullptr, *d_passq = nullptr;
-    int64_t cap_frames = 0, cap_cand = 0, cap_passq = 0, n_cand_last = 0;
-    mcx_hit *d_hsp = nullptr, *d_hits_out = nullptr;
-    SortKey *d_keys = nullptr;
-    int32_t *d_idx = nullptr, *d_best = nullptr, *d_hflag = nullptr, *d_hpos = nullptr;
-    uint8_t *d_keep = nullptr;
-    int32_t *d_nrep = nullptr;
-    unsigned long long *d_bestkey = nullptr;
-    int64_t cap_surv = 0, cap_best = 0, cap_nrep = 0, cap_bestkey = 0;
-    unsigned long long *d_cnt = nullptr;     // 64 scalar counters (layout: enum Cnt)
-    int n_sm = 148;                          // multiprocessors of the device (sizes the resident grids)
-    unsigned long long *d_qcnt = nullptr;    // NQ candidate sub-queue fills, then NQ filter-pass sub-queue fills
-    unsigned long long *d_acc = nullptr;     // 3 + 60
-    unsigned long long *d_abl = nullptr;     // 30 * 1280
-    unsigned long long *h_cnt = nullptr;     // pinned mirror for counter read-backs (64 + NQ)
-    void *d_temp = nullptr;
-    size_t temp_bytes = 0;
-    int64_t n_hsp_sorted = 0;
+    DevBuf<uint4> d_surv;
+    DevBuf<uint8_t> d_frames;
+    DevBuf<uint32_t> d_segq, d_segm;
+    DevBuf<unsigned long long> d_seen;         // k_walk's duplicate filter
+    DevBuf<uint4> d_seedq;                     // accepted seeds between k_seed and k_walk
+    DevBuf<unsigned long long> d_gitems;       // gapped work lists: three regions of 2 * survivors entries
+    DevBuf<GExtRec> d_gext;
+    DevBuf<uint32_t> d_dirs;                   // direction nibbles of k_gap_dp for k_gap_trace
+    DevBuf<Cand> d_cand, d_passq;
+    DevBuf<mcx_hit> d_hsp, d_hits_out;
+    DevBuf<SortKey> d_keys;
+    DevBuf<int32_t> d_idx, d_best, d_hflag, d_hpos;
+    DevBuf<uint8_t> d_keep;
+    DevBuf<int32_t> d_nrep;
+    DevBuf<unsigned long long> d_bestkey;
+    DevBuf<unsigned long long> d_cnt;          // 64 scalar counters (layout: enum Cnt)
+    int n_sm = 148;                            // multiprocessors of the device (sizes the resident grids)
+    DevBuf<unsigned long long> d_qcnt;         // NQ candidate sub-queue fills, then NQ filter-pass sub-queue fills
+    DevBuf<unsigned long long> d_acc;          // 3 + 60
+    DevBuf<unsigned long long> d_abl;          // 30 * 1280
+    unsigned long long *h_cnt = nullptr;       // pinned mirror for counter read-backs (64 + NQ)
+    DevBuf<uint8_t> d_temp;                    // CUB's temporary storage (cub_run)
     mcx_result res{};
-    float ms[12] = {0};
-    float ms_detail[4] = {0};                  // k_probe, k_resolve, k_seed, k_walk of the last search
+    float ms[MS_N] = {0};
+    float ms_detail[MSD_N] = {0};
     int64_t work[8] = {0};                     // mcx_search_counters of the last search
     int64_t launches = 0, host_syncs = 0;
-    cudaEvent_t ev[22] = {nullptr};
+    cudaEvent_t ev[EV_N] = {nullptr};
 };
 // slots of d_cnt
 enum Cnt { C_QC0 = 0 /* ..3: verdict counts of the search */, C_QCALL = 4 /* ..7: verdict counts over all pushed reads */,
@@ -2401,59 +2446,50 @@ static int fail(mcx_ctx *ctx, int code, const std::string &msg) {
     g_err = msg;
     return code;
 }
-#define CK(call)                                                                                   \
-    do {                                                                                           \
-        cudaError_t e_ = (call);                                                                   \
-        if (e_ != cudaSuccess)                                                                     \
-            return fail(ctx, MCX_ECUDA, std::string(#call) + ": " + cudaGetErrorString(e_));       \
-    } while (0)
 
 template <typename T>
-static cudaError_t dev_alloc(T **p, size_t n) { return cudaMalloc((void **)p, n * sizeof(T) ? n * sizeof(T) : 1); }
-
-template <typename T>
-static int ensure(mcx_ctx *ctx, T **p, int64_t *cap, int64_t need) {
-    if (*cap >= need && *p) return MCX_OK;
-    if (*p) CK(cudaFree(*p));
-    *p = nullptr;
-    int64_t c = need + need / 8 + 16;
-    CK(dev_alloc(p, (size_t)c));
-    *cap = c;
-    return MCX_OK;
-}
-
-template <typename T>
-static int grow_keep(mcx_ctx *ctx, T **p, int64_t keep, int64_t cap) {
+int DevBuf<T>::grow_keep(mcx_ctx *ctx, int64_t keep, int64_t c) {
     T *q = nullptr;
-    CK(dev_alloc(&q, (size_t)cap));
-    if (*p && keep > 0) CK(cudaMemcpyAsync(q, *p, (size_t)keep * sizeof(T), cudaMemcpyDeviceToDevice, ctx->stream));
+    CK(dev_alloc(&q, (size_t)c));
+    if (p && keep > 0) CK(cudaMemcpyAsync(q, p, (size_t)keep * sizeof(T), cudaMemcpyDeviceToDevice, ctx->stream));
     CK(cudaStreamSynchronize(ctx->stream));
-    if (*p) CK(cudaFree(*p));
-    *p = q;
+    TRY(release(ctx));
+    p = q; cap = c;
     return MCX_OK;
 }
 
 // survivor-sized buffers: keep the first `keep` entries of the ones that carry state across chunks
 static int grow_survivors(mcx_ctx *ctx, int64_t keep, int64_t cap) {
-    int rc;
-    if ((rc = grow_keep(ctx, &ctx->d_surv, keep, cap)) != MCX_OK) return rc;
-    if ((rc = grow_keep(ctx, &ctx->d_hsp, keep, cap)) != MCX_OK) return rc;
-    if ((rc = grow_keep(ctx, &ctx->d_keys, keep, cap)) != MCX_OK) return rc;
-    if ((rc = grow_keep(ctx, &ctx->d_idx, keep, cap)) != MCX_OK) return rc;
-    if ((rc = grow_keep(ctx, &ctx->d_hits_out, 0, cap)) != MCX_OK) return rc;
-    if ((rc = grow_keep(ctx, &ctx->d_hflag, 0, cap + 1)) != MCX_OK) return rc;
-    if ((rc = grow_keep(ctx, &ctx->d_hpos, 0, cap + 1)) != MCX_OK) return rc;
-    if ((rc = grow_keep(ctx, &ctx->d_keep, 0, cap)) != MCX_OK) return rc;
-    ctx->cap_surv = cap;
+    TRY(ctx->d_surv.grow_keep(ctx, keep, cap));
+    TRY(ctx->d_hsp.grow_keep(ctx, keep, cap));
+    TRY(ctx->d_keys.grow_keep(ctx, keep, cap));
+    TRY(ctx->d_idx.grow_keep(ctx, keep, cap));
+    TRY(ctx->d_hits_out.grow_keep(ctx, 0, cap));
+    TRY(ctx->d_hflag.grow_keep(ctx, 0, cap + 1));
+    TRY(ctx->d_hpos.grow_keep(ctx, 0, cap + 1));
+    TRY(ctx->d_keep.grow_keep(ctx, 0, cap));
     return MCX_OK;
 }
 
-static int ensure_temp(mcx_ctx *ctx, size_t bytes) {
-    if (ctx->temp_bytes >= bytes && ctx->d_temp) return MCX_OK;
-    if (ctx->d_temp) CK(cudaFree(ctx->d_temp));
-    ctx->d_temp = nullptr;
-    CK(cudaMalloc(&ctx->d_temp, bytes + bytes / 8 + 256));
-    ctx->temp_bytes = bytes + bytes / 8 + 256;
+// a CUB call in its two phases: the temporary storage it asks for, then the call itself on ctx->d_temp
+template <typename F>
+static int cub_run(mcx_ctx *ctx, const char *what, F call) {
+    size_t tb = 0;
+    cudaError_t e = call(nullptr, tb);
+    if (e == cudaSuccess) {
+        TRY(ctx->d_temp.ensure(ctx, (int64_t)tb, nullptr, 256));
+        e = call(ctx->d_temp.p, tb);
+    }
+    if (e != cudaSuccess) return fail(ctx, MCX_ECUDA, std::string(what) + ": " + cudaGetErrorString(e));
+    return MCX_OK;
+}
+
+// blocks of `kernel` that are resident on the device at once (at least one per multiprocessor)
+template <typename K>
+static int resident_blocks(mcx_ctx *ctx, K kernel, int nt, size_t smem, unsigned &blocks) {
+    int per_sm = 0;
+    CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, nt, smem));
+    blocks = (unsigned)(std::max(per_sm, 1) * ctx->n_sm);
     return MCX_OK;
 }
 
@@ -2584,6 +2620,97 @@ static int build_index(mcx_ctx *ctx, const mcx_db *db) {
     return MCX_OK;
 }
 
+// every way of writing tot as at most 20 letter counts, largest first (the order seg.c sums them in): f(counts, n)
+template <typename F>
+static void for_each_partition(int tot, F f) {
+    int part[20];
+    auto rec = [&](auto &&self, int left, int maxpart, int np) -> void {
+        if (left == 0) return f((const int *)part, np);
+        if (np == 20) return;
+        for (int k = std::min(left, maxpart); k >= 1; --k) { part[np] = k; self(self, left - k, k, np + 1); }
+    };
+    rec(rec, tot, tot, 0);
+}
+
+// the two SEG tables: the integer window test and getprob() of every window class
+static int upload_seg_tables(mcx_ctx *ctx, const double *lnfac, const double *ln20, const double *ent) {
+    // integer form of the SEG window test (see SegTab): thresholds taken from the reference's own double sums
+    SegTab T;
+    memset(&T, 0, sizeof T);
+    long long gfix[13];
+    gfix[0] = 0;
+    for (int c = 1; c <= SEG_WINDOW; ++c) gfix[c] = llround((double)c * log2((double)c) * 16777216.0);
+    for (int c = 0; c < SEG_WINDOW; ++c) T.dg[c] = (int)(gfix[c + 1] - gfix[c]);
+    for (int tot = 0; tot <= SEG_WINDOW; ++tot) {
+        long long min_yes[2] = {LLONG_MAX, LLONG_MAX}, max_no[2] = {LLONG_MIN, LLONG_MIN};
+        for_each_partition(tot, [&](const int *part, int np) {
+            double e = 0.0;
+            long long G = 0;
+            for (int k = 0; k < np; ++k) { e += ent[tot * 13 + part[k]]; G += gfix[part[k]]; }
+            const double cut[2] = {SEG_LOCUT, SEG_HICUT};
+            for (int q = 0; q < 2; ++q) {
+                if (e <= cut[q]) min_yes[q] = std::min(min_yes[q], G);
+                else max_no[q] = std::max(max_no[q], G);
+            }
+        });
+        for (int q = 0; q < 2; ++q)
+            if (max_no[q] >= min_yes[q]) return fail(ctx, MCX_EINVAL, "internal: integer SEG window test does not separate the entropy cut-offs");
+        T.thr[tot].x = (int)std::min<long long>(min_yes[0], INT_MAX);
+        T.thr[tot].y = (int)std::min<long long>(min_yes[1], INT_MAX);
+    }
+    CK(cudaMemcpyToSymbol(g_segtab, &T, sizeof T));
+    // getprob() of every (window length <= 20, multiset of letter counts), see g_segprob
+    uint32_t z[32] = {0};
+    std::vector<SegProbSlot> tab;
+    for (unsigned long long seed = 0x243F6A8885A308D3ull;; seed += 0x9E3779B97F4A7C15ull) {
+        unsigned long long x = seed;
+        z[0] = 0;
+        for (int c = 1; c <= SEGP_MAXLEN; ++c) {         // splitmix64
+            x += 0x9E3779B97F4A7C15ull;
+            unsigned long long t = x;
+            t = (t ^ (t >> 30)) * 0xBF58476D1CE4E5B9ull; t = (t ^ (t >> 27)) * 0x94D049BB133111EBull; t ^= t >> 31;
+            z[c] = (uint32_t)t;
+        }
+        tab.assign(SEGP_SLOTS, SegProbSlot{~0ull, 0.0});
+        bool unique = true;
+        size_t classes = 0;
+        for (int len = 1; len <= SEGP_MAXLEN && unique; ++len)
+            for (int tot = 0; tot <= len && unique; ++tot)
+                for_each_partition(tot, [&](const int *part, int np) {
+                    if (!unique) return;
+                    // seg.c getprob() on the counts, largest first (same operations as seg_getprob above)
+                    double lnperm = lnfac[len], lnass = lnfac[20];
+                    uint32_t sig = 0;
+                    int nz = 0;
+                    for (int k = 0; k < np;) {
+                        int e = k;
+                        while (e + 1 < np && part[e + 1] == part[k]) ++e;
+                        const int c = part[k], n = e - k + 1;
+                        if (c > 1) for (int r = 0; r < n; ++r) lnperm -= lnfac[c];
+                        if (n > 1) lnass -= lnfac[n];
+                        nz += n;
+                        sig += (uint32_t)n * z[c];
+                        k = e + 1;
+                    }
+                    if (nz > 0 && nz < 20) lnass -= lnfac[20 - nz];
+                    const double prob = lnass + lnperm - ln20[len];
+                    const unsigned long long key = ((unsigned long long)len << 32) | sig;
+                    uint32_t sl = segp_slot(key);
+                    while (tab[sl].key != ~0ull) {
+                        if (tab[sl].key == key) { unique = false; return; }
+                        sl = (sl + 1) & (SEGP_SLOTS - 1);
+                    }
+                    tab[sl] = SegProbSlot{key, prob};
+                    ++classes;
+                });
+        if (unique && classes * 2 <= (size_t)SEGP_SLOTS) break;
+        if (classes * 2 > (size_t)SEGP_SLOTS) return fail(ctx, MCX_EINVAL, "internal: SEG probability table too small");
+    }
+    CK(cudaMemcpyToSymbol(g_segz, z, sizeof z));
+    CK(cudaMemcpyToSymbol(g_segprob, tab.data(), sizeof(SegProbSlot) * SEGP_SLOTS));
+    return MCX_OK;
+}
+
 static int upload_tables(mcx_ctx *ctx) {
     double lnfac[256], ln20[256], ent[13 * 13];
     for (int i = 0; i < 256; ++i) { lnfac[i] = lgamma((double)i + 1.0); ln20[i] = (double)i * log(20.0); }
@@ -2599,100 +2726,7 @@ static int upload_tables(mcx_ctx *ctx) {
         const char *p = strchr(AA_ORDER, CODON_AA[i]);
         codon[i] = (p && CODON_AA[i] != '.') ? (uint8_t)(p - AA_ORDER) : (uint8_t)AA_STOP;
     }
-    // integer form of the SEG window test (see SegTab): thresholds taken from the reference's own double sums
-    {
-        SegTab T;
-        memset(&T, 0, sizeof T);
-        long long gfix[13];
-        gfix[0] = 0;
-        for (int c = 1; c <= SEG_WINDOW; ++c) gfix[c] = llround((double)c * log2((double)c) * 16777216.0);
-        for (int c = 0; c < SEG_WINDOW; ++c) T.dg[c] = (int)(gfix[c + 1] - gfix[c]);
-        for (int tot = 0; tot <= SEG_WINDOW; ++tot) {
-            long long min_yes[2] = {LLONG_MAX, LLONG_MAX}, max_no[2] = {LLONG_MIN, LLONG_MIN};
-            int part[20];
-            // every way of writing tot as at most 20 letter counts, largest first (the order seg.c sums them in)
-            auto rec = [&](auto &&self, int left, int maxpart, int np) -> void {
-                if (left == 0) {
-                    double e = 0.0;
-                    long long G = 0;
-                    for (int k = 0; k < np; ++k) { e += ent[tot * 13 + part[k]]; G += gfix[part[k]]; }
-                    const double cut[2] = {SEG_LOCUT, SEG_HICUT};
-                    for (int q = 0; q < 2; ++q) {
-                        if (e <= cut[q]) min_yes[q] = std::min(min_yes[q], G);
-                        else max_no[q] = std::max(max_no[q], G);
-                    }
-                    return;
-                }
-                if (np == 20) return;
-                for (int k = std::min(left, maxpart); k >= 1; --k) { part[np] = k; self(self, left - k, k, np + 1); }
-            };
-            rec(rec, tot, tot, 0);
-            for (int q = 0; q < 2; ++q)
-                if (max_no[q] >= min_yes[q]) return fail(ctx, MCX_EINVAL, "internal: integer SEG window test does not separate the entropy cut-offs");
-            T.thr[tot].x = (int)std::min<long long>(min_yes[0], INT_MAX);
-            T.thr[tot].y = (int)std::min<long long>(min_yes[1], INT_MAX);
-        }
-        CK(cudaMemcpyToSymbol(g_segtab, &T, sizeof T));
-    }
-    // getprob() of every (window length <= 20, multiset of letter counts), see g_segprob
-    {
-        uint32_t z[32] = {0};
-        std::vector<SegProbSlot> tab;
-        for (unsigned long long seed = 0x243F6A8885A308D3ull;; seed += 0x9E3779B97F4A7C15ull) {
-            unsigned long long x = seed;
-            z[0] = 0;
-            for (int c = 1; c <= SEGP_MAXLEN; ++c) {         // splitmix64
-                x += 0x9E3779B97F4A7C15ull;
-                unsigned long long t = x;
-                t = (t ^ (t >> 30)) * 0xBF58476D1CE4E5B9ull; t = (t ^ (t >> 27)) * 0x94D049BB133111EBull; t ^= t >> 31;
-                z[c] = (uint32_t)t;
-            }
-            tab.assign(SEGP_SLOTS, SegProbSlot{~0ull, 0.0});
-            bool unique = true;
-            size_t classes = 0;
-            int part[20];
-            for (int len = 1; len <= SEGP_MAXLEN && unique; ++len)
-                for (int tot = 0; tot <= len && unique; ++tot) {
-                    auto rec = [&](auto &&self, int left, int maxpart, int np) -> void {
-                        if (!unique) return;
-                        if (left == 0) {
-                            // seg.c getprob() on the counts, largest first (same operations as seg_getprob above)
-                            double lnperm = lnfac[len], lnass = lnfac[20];
-                            uint32_t sig = 0;
-                            int nz = 0;
-                            for (int k = 0; k < np;) {
-                                int e = k;
-                                while (e + 1 < np && part[e + 1] == part[k]) ++e;
-                                const int c = part[k], n = e - k + 1;
-                                if (c > 1) for (int r = 0; r < n; ++r) lnperm -= lnfac[c];
-                                if (n > 1) lnass -= lnfac[n];
-                                nz += n;
-                                sig += (uint32_t)n * z[c];
-                                k = e + 1;
-                            }
-                            if (nz > 0 && nz < 20) lnass -= lnfac[20 - nz];
-                            const double prob = lnass + lnperm - ln20[len];
-                            const unsigned long long key = ((unsigned long long)len << 32) | sig;
-                            uint32_t sl = segp_slot(key);
-                            while (tab[sl].key != ~0ull) {
-                                if (tab[sl].key == key) { unique = false; return; }
-                                sl = (sl + 1) & (SEGP_SLOTS - 1);
-                            }
-                            tab[sl] = SegProbSlot{key, prob};
-                            ++classes;
-                            return;
-                        }
-                        if (np == 20) return;
-                        for (int k = std::min(left, maxpart); k >= 1; --k) { part[np] = k; self(self, left - k, k, np + 1); }
-                    };
-                    rec(rec, tot, tot, 0);
-                }
-            if (unique && classes * 2 <= (size_t)SEGP_SLOTS) break;
-            if (classes * 2 > (size_t)SEGP_SLOTS) return fail(ctx, MCX_EINVAL, "internal: SEG probability table too small");
-        }
-        CK(cudaMemcpyToSymbol(g_segz, z, sizeof z));
-        CK(cudaMemcpyToSymbol(g_segprob, tab.data(), sizeof(SegProbSlot) * SEGP_SLOTS));
-    }
+    TRY(upload_seg_tables(ctx, lnfac, ln20, ent));
     {
         uint8_t lut[256];
         memset(lut, AA_STOP, sizeof lut);
@@ -2741,7 +2775,6 @@ extern "C" int mcx_create(mcx_ctx **out, const mcx_db *db, int device) {
     if (device < 0 || device >= ndev) return fail(nullptr, MCX_EINVAL, "mcx_create: device index out of range");
     mcx_ctx *ctx = new mcx_ctx();
     ctx->device = device;
-    int rc = MCX_OK;
     auto body = [&]() -> int {
         CK(cudaSetDevice(device));
         CK(cudaDeviceGetAttribute(&ctx->n_sm, cudaDevAttrMultiProcessorCount, device));
@@ -2749,8 +2782,6 @@ extern "C" int mcx_create(mcx_ctx **out, const mcx_db *db, int device) {
         CK(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
         for (auto &ev : ctx->ev) CK(cudaEventCreate(&ev));
         for (auto &ev : ctx->ev_copy) CK(cudaEventCreateWithFlags(&ev, cudaEventDisableTiming));
-        CK(cudaEventCreateWithFlags(&ctx->ev_len, cudaEventDisableTiming));
-        CK(cudaEventCreate(&ctx->ev_h2d0));
         CK(cudaHostAlloc((void **)&ctx->h_cnt, (C_N + 2 * NQ) * sizeof(unsigned long long), cudaHostAllocDefault));
         const int ns = db->n_subj;
         const int64_t nres = db->off[ns];
@@ -2764,16 +2795,15 @@ extern "C" int mcx_create(mcx_ctx **out, const mcx_db *db, int device) {
         CK(cudaMemcpy(dres, db->res, (size_t)nres, cudaMemcpyHostToDevice));
         CK(cudaMemcpy(dfam, db->fam, (size_t)ns, cudaMemcpyHostToDevice));
         ctx->db.n_subj = ns; ctx->db.off = doff; ctx->db.res = dres; ctx->db.fam = dfam;
-        ctx->n_subj = ns;
-        int r = upload_tables(ctx); if (r) return r;
-        r = build_index(ctx, db); if (r) return r;
-        CK(dev_alloc(&ctx->d_cnt, C_N));
-        CK(dev_alloc(&ctx->d_qcnt, 2 * NQ));
-        CK(dev_alloc(&ctx->d_acc, 3 + 2 * MCX_N_FAM));
-        CK(dev_alloc(&ctx->d_abl, (size_t)MCX_N_FAM * MCX_LEN_BINS));
+        TRY(upload_tables(ctx));
+        TRY(build_index(ctx, db));
+        TRY(ctx->d_cnt.ensure(ctx, C_N));
+        TRY(ctx->d_qcnt.ensure(ctx, 2 * NQ));
+        TRY(ctx->d_acc.ensure(ctx, 3 + 2 * MCX_N_FAM));
+        TRY(ctx->d_abl.ensure(ctx, (int64_t)MCX_N_FAM * MCX_LEN_BINS));
         return MCX_OK;
     };
-    rc = body();
+    const int rc = body();
     if (rc != MCX_OK) { g_err = ctx->err; mcx_destroy(ctx); return rc; }
     *out = ctx;
     return MCX_OK;
@@ -2784,22 +2814,12 @@ extern "C" void mcx_destroy(mcx_ctx *ctx) {
     cudaSetDevice(ctx->device);
     cudaDeviceSynchronize();
     for (void *p : ctx->db_allocs) cudaFree(p);
-    if (!ctx->ext_pk) cudaFree(ctx->d_pk);
-    if (!ctx->ext_len) cudaFree(ctx->d_len);
-    if (!ctx->ext_quals) cudaFree(ctx->d_quals);
-    void *bufs[] = {ctx->d_woff, ctx->d_qoff, ctx->d_ascii, ctx->d_aoffs, ctx->d_code, ctx->d_fp, ctx->d_fpa, ctx->d_fpa2, ctx->d_fpi, ctx->d_fpi2,
-                    ctx->d_kept, ctx->d_store_a, ctx->d_store_b, ctx->d_xsend, ctx->d_xmarks, ctx->d_xkg, ctx->d_xvi, ctx->d_surv, ctx->d_hsp, ctx->d_hits_out, ctx->d_keys, ctx->d_idx, ctx->d_best, ctx->d_hflag,
-                    ctx->d_hpos, ctx->d_keep, ctx->d_cnt, ctx->d_acc, ctx->d_abl, ctx->d_temp, ctx->d_frames, ctx->d_cand,
-                    ctx->d_segq, ctx->d_segm, ctx->d_passq, ctx->d_qcnt, ctx->d_gitems, ctx->d_gext, ctx->d_dirs, ctx->d_nrep, ctx->d_bestkey, ctx->d_seen, ctx->d_seedq};
-    for (void *p : bufs) if (p) cudaFree(p);
     if (ctx->h_cnt) cudaFreeHost(ctx->h_cnt);
     for (auto &ev : ctx->ev) if (ev) cudaEventDestroy(ev);
     for (auto &ev : ctx->ev_copy) if (ev) cudaEventDestroy(ev);
-    if (ctx->ev_len) cudaEventDestroy(ctx->ev_len);
-    if (ctx->ev_h2d0) cudaEventDestroy(ctx->ev_h2d0);
     if (ctx->copy_stream) cudaStreamDestroy(ctx->copy_stream);
     if (ctx->stream && ctx->own_stream) cudaStreamDestroy(ctx->stream);
-    delete ctx;
+    delete ctx;                                   // the DevBuf members free their storage
 }
 
 extern "C" int mcx_set_stream(mcx_ctx *ctx, void *cuda_stream) {
@@ -2831,55 +2851,49 @@ extern "C" int mcx_set_params(mcx_ctx *ctx, const mcx_params *p) {
 static ReadStore read_store(const mcx_ctx *ctx) {
     ReadStore S;
     S.pk = ctx->d_pk; S.woff = ctx->d_woff; S.len = ctx->d_len;
-    S.quals = (ctx->have_quals && ctx->par.has_quality) ? ctx->d_quals : nullptr;
+    S.quals = (ctx->have_quals && ctx->par.has_quality) ? ctx->d_quals.p : nullptr;
     S.qoff = ctx->d_qoff; S.qbytes = ctx->n_bases;
     return S;
-}
-
-static void release_external(mcx_ctx *ctx) {      // forget caller-owned buffers of an earlier *_dev push
-    if (ctx->ext_pk) { ctx->d_pk = nullptr; ctx->cap_pk = 0; ctx->ext_pk = false; }
-    if (ctx->ext_len) { ctx->d_len = nullptr; ctx->cap_len = 0; ctx->ext_len = false; }
-    if (ctx->ext_quals) { ctx->d_quals = nullptr; ctx->cap_quals = 0; ctx->ext_quals = false; }
 }
 
 // offsets of the records and of the qualities from the lengths (two scans over n + 1 items: slot n receives the total)
 static int scan_offsets(mcx_ctx *ctx, bool with_quals) {
     const int64_t n = ctx->n_reads;
     cudaStream_t st = ctx->stream;
-    int rc;
-    if ((rc = ensure(ctx, &ctx->d_woff, &ctx->cap_woff, n + 1)) != MCX_OK) return rc;
-    if (with_quals && (rc = ensure(ctx, &ctx->d_qoff, &ctx->cap_qoff, n + 1)) != MCX_OK) return rc;
-    auto gw = thrust::make_transform_iterator(static_cast<const uint32_t *>(ctx->d_len), GroupsOf());
-    auto gl = thrust::make_transform_iterator(static_cast<const uint32_t *>(ctx->d_len), LenOf());
-    size_t tb = 0, tb2 = 0;
-    CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, gw, ctx->d_woff, (int)(n + 1), st));
-    CK(cub::DeviceScan::ExclusiveSum(nullptr, tb2, gl, ctx->d_qoff, (int)(n + 1), st));
-    if ((rc = ensure_temp(ctx, std::max(tb, tb2))) != MCX_OK) return rc;
-    CK(cub::DeviceScan::ExclusiveSum(ctx->d_temp, tb, gw, ctx->d_woff, (int)(n + 1), st));
+    TRY(ctx->d_woff.ensure(ctx, n + 1));
+    if (with_quals) TRY(ctx->d_qoff.ensure(ctx, n + 1));
+    auto gw = thrust::make_transform_iterator(static_cast<const uint32_t *>(ctx->d_len.p), GroupsOf());
+    auto gl = thrust::make_transform_iterator(static_cast<const uint32_t *>(ctx->d_len.p), LenOf());
+    TRY(cub_run(ctx, "cub::DeviceScan::ExclusiveSum (record offsets)", [&](void *t, size_t &tb) {
+        return cub::DeviceScan::ExclusiveSum(t, tb, gw, ctx->d_woff.p, (int)(n + 1), st); }));
     ctx->launches += 2;
-    if (with_quals) { CK(cub::DeviceScan::ExclusiveSum(ctx->d_temp, tb2, gl, ctx->d_qoff, (int)(n + 1), st)); ctx->launches += 2; }
+    if (with_quals) {
+        TRY(cub_run(ctx, "cub::DeviceScan::ExclusiveSum (quality offsets)", [&](void *t, size_t &tb) {
+            return cub::DeviceScan::ExclusiveSum(t, tb, gl, ctx->d_qoff.p, (int)(n + 1), st); }));
+        ctx->launches += 2;
+    }
     return MCX_OK;
 }
 
-static int begin_push(mcx_ctx *ctx, const char *who, int64_t n, bool quals_given) {
+// n_words < 0: not known on the host (ASCII reads are packed on the device; nothing waits on copy steps then)
+static int begin_push(mcx_ctx *ctx, const char *who, int64_t n, int64_t n_words, int64_t n_bases, const void *quals) {
     if (!ctx->have_par) return fail(ctx, MCX_ESTATE, std::string(who) + ": call mcx_set_params first");
     if (n >= (1ll << 27)) return fail(ctx, MCX_EINVAL, std::string(who) + ": at most 2^27 reads per call");
-    if (ctx->par.has_quality && !quals_given && n > 0) return fail(ctx, MCX_EINVAL, std::string(who) + ": FASTQ parameters but no qualities");
+    if (ctx->par.has_quality && !quals && n > 0) return fail(ctx, MCX_EINVAL, std::string(who) + ": FASTQ parameters but no qualities");
     CK(cudaSetDevice(ctx->device));
-    release_external(ctx);
     ctx->launches = 0; ctx->host_syncs = 0;
     memset(ctx->ms, 0, sizeof ctx->ms);
     (void)cudaGetLastError();                  // nothing an earlier call left behind may stop CUB's dispatches
     ctx->n_steps = 0; ctx->steps_waited = 0; ctx->h2d_timed = false;
     ctx->qc_upto = 0; ctx->dedup_done = false; ctx->fp_done = false; ctx->counts_valid = false;
     ctx->pushed = false; ctx->searched = false;
+    ctx->n_reads = n; ctx->n_words = n_words; ctx->n_bases = n_bases; ctx->have_quals = quals != nullptr;
     return MCX_OK;
 }
 
 static int end_push(mcx_ctx *ctx) {
-    int rc;
     const int64_t n = ctx->n_reads;
-    if ((rc = ensure(ctx, &ctx->d_code, &ctx->cap_code, n + 1)) != MCX_OK) return rc;
+    TRY(ctx->d_code.ensure(ctx, n + 1));
     CK(cudaMemsetAsync(ctx->d_code, 4, (size_t)(n + 1), ctx->stream));       // 4 = not examined
     ctx->pushed = true;
     return MCX_OK;
@@ -2896,19 +2910,17 @@ extern "C" int mcx_push_reads_packed(mcx_ctx *ctx, const uint32_t *packed, int64
                                      const uint8_t *quals, int64_t n_bases, int64_t n) {
     if (!ctx || n < 0 || n_words < 0 || n_bases < 0 || (n > 0 && (!packed || !lengths)))
         return fail(ctx, MCX_EINVAL, "mcx_push_reads_packed: bad argument");
-    int rc;
-    if ((rc = begin_push(ctx, "mcx_push_reads_packed", n, quals != nullptr)) != MCX_OK) return rc;
-    ctx->n_reads = n; ctx->n_words = n_words; ctx->n_bases = n_bases; ctx->have_quals = quals != nullptr;
-    if ((rc = ensure(ctx, &ctx->d_pk, &ctx->cap_pk, n_words + 4)) != MCX_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_len, &ctx->cap_len, n + 1)) != MCX_OK) return rc;
-    if (quals && (rc = ensure(ctx, &ctx->d_quals, &ctx->cap_quals, n_bases + 32)) != MCX_OK) return rc;
+    TRY(begin_push(ctx, "mcx_push_reads_packed", n, n_words, n_bases, quals));
+    TRY(ctx->d_pk.ensure(ctx, n_words + 4));
+    TRY(ctx->d_len.ensure(ctx, n + 1));
+    if (quals) TRY(ctx->d_quals.ensure(ctx, n_bases + 32));
     cudaStream_t cs = ctx->copy_stream;
     // the copies run on their own stream in steps, an event behind each; the search waits per chunk of reads for
     // the steps that hold it, so the copy of later reads overlaps the kernels of earlier ones
-    CK(cudaEventRecord(ctx->ev_h2d0, cs));
+    CK(cudaEventRecord(ctx->ev[EV_H2D0], cs));
     if (n > 0) CK(cudaMemcpyAsync(ctx->d_len, lengths, (size_t)n * sizeof(uint32_t), cudaMemcpyHostToDevice, cs));
     CK(cudaMemsetAsync(ctx->d_len + n, 0, sizeof(uint32_t), cs));
-    CK(cudaEventRecord(ctx->ev_len, cs));
+    CK(cudaEventRecord(ctx->ev[EV_LENS], cs));
     const int K = copy_steps(n_words * 4 + (quals ? n_bases : 0));
     ctx->step_words = (n_words + K - 1) / K;
     ctx->step_qbytes = (((n_bases + K - 1) / K) + 15) & ~15ll;
@@ -2921,10 +2933,10 @@ extern "C" int mcx_push_reads_packed(mcx_ctx *ctx, const uint32_t *packed, int64
         }
         CK(cudaEventRecord(ctx->ev_copy[k], cs));
     }
-    CK(cudaEventRecord(ctx->ev[19], cs));
+    CK(cudaEventRecord(ctx->ev[EV_H2D1], cs));
     ctx->n_steps = K; ctx->h2d_timed = true;
-    CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_len, 0));
-    if ((rc = scan_offsets(ctx, quals != nullptr)) != MCX_OK) return rc;
+    CK(cudaStreamWaitEvent(ctx->stream, ctx->ev[EV_LENS], 0));
+    TRY(scan_offsets(ctx, quals != nullptr));
     return end_push(ctx);
 }
 
@@ -2933,67 +2945,51 @@ extern "C" int mcx_push_reads_packed_dev(mcx_ctx *ctx, const uint32_t *d_packed,
     if (!ctx || n < 0 || n_words < 0 || n_bases < 0 || (n > 0 && (!d_packed || !d_lengths)))
         return fail(ctx, MCX_EINVAL, "mcx_push_reads_packed_dev: bad argument");
     if (d_quals && ((uintptr_t)d_quals & 15)) return fail(ctx, MCX_EINVAL, "mcx_push_reads_packed_dev: qualities must be 16-byte aligned");
-    int rc;
-    if ((rc = begin_push(ctx, "mcx_push_reads_packed_dev", n, d_quals != nullptr)) != MCX_OK) return rc;
-    ctx->n_reads = n; ctx->n_words = n_words; ctx->n_bases = n_bases; ctx->have_quals = d_quals != nullptr;
-    if (!ctx->ext_pk && ctx->d_pk) { CK(cudaFree(ctx->d_pk)); }
-    if (!ctx->ext_quals && ctx->d_quals) { CK(cudaFree(ctx->d_quals)); }
-    ctx->d_pk = const_cast<uint32_t *>(d_packed); ctx->ext_pk = true; ctx->cap_pk = 0;
-    ctx->d_quals = const_cast<uint8_t *>(d_quals); ctx->ext_quals = true; ctx->cap_quals = 0;
+    TRY(begin_push(ctx, "mcx_push_reads_packed_dev", n, n_words, n_bases, d_quals));
+    TRY(ctx->d_pk.borrow(ctx, const_cast<uint32_t *>(d_packed)));
+    TRY(ctx->d_quals.borrow(ctx, const_cast<uint8_t *>(d_quals)));
     // the lengths are copied (n + 1 entries are scanned; the caller's array has n)
-    if ((rc = ensure(ctx, &ctx->d_len, &ctx->cap_len, n + 1)) != MCX_OK) return rc;
+    TRY(ctx->d_len.ensure(ctx, n + 1));
     if (n > 0) CK(cudaMemcpyAsync(ctx->d_len, d_lengths, (size_t)n * sizeof(uint32_t), cudaMemcpyDeviceToDevice, ctx->stream));
     CK(cudaMemsetAsync(ctx->d_len + n, 0, sizeof(uint32_t), ctx->stream));
-    if ((rc = scan_offsets(ctx, d_quals != nullptr)) != MCX_OK) return rc;
+    TRY(scan_offsets(ctx, d_quals != nullptr));
     return end_push(ctx);
 }
 
-// ASCII reads (device-resident by now): lengths, offsets, then the bit-planes
-static int pack_ascii(mcx_ctx *ctx, const uint8_t *d_bases, const int64_t *d_offsets, int64_t n, int64_t total, bool with_quals) {
+// ASCII reads (device-resident by now): lengths, offsets, bit-planes; the qualities take the offsets of the bases
+static int pack_ascii(mcx_ctx *ctx, const uint8_t *d_bases, const int64_t *d_offsets, int64_t n, int64_t total) {
     cudaStream_t st = ctx->stream;
-    int rc;
-    if ((rc = ensure(ctx, &ctx->d_len, &ctx->cap_len, n + 1)) != MCX_OK) return rc;
+    TRY(ctx->d_len.ensure(ctx, n + 1));
     k_lens_from_offsets<<<(unsigned)((n + 1 + 255) / 256), 256, 0, st>>>(d_offsets, n, ctx->d_len);
-    if ((rc = scan_offsets(ctx, false)) != MCX_OK) return rc;
+    TRY(scan_offsets(ctx, false));
     // every read of l bases takes 3 ceil(l / 32) words: at most 3 (total / 32 + n)
     const int64_t bound = 3 * (total / 32 + n) + 4;
-    if ((rc = ensure(ctx, &ctx->d_pk, &ctx->cap_pk, bound)) != MCX_OK) return rc;
+    TRY(ctx->d_pk.ensure(ctx, bound));
     if (n > 0) k_pack_ascii<<<(unsigned)((n * 32 + 255) / 256), 256, 0, st>>>(d_bases, d_offsets, n, ctx->d_woff, ctx->d_pk);
     ctx->launches += 2;
-    if (getenv("MCX_DEBUG_PACK")) {
-        long long w[3] = {0, 0, 0}; uint32_t l0 = 0, p0[4] = {0, 0, 0, 0};
-        cudaMemcpy(&w[0], ctx->d_woff + 1, 8, cudaMemcpyDeviceToHost); cudaMemcpy(&w[1], ctx->d_woff + n, 8, cudaMemcpyDeviceToHost);
-        cudaMemcpy(&l0, ctx->d_len, 4, cudaMemcpyDeviceToHost); cudaMemcpy(p0, ctx->d_pk + w[0], 16, cudaMemcpyDeviceToHost);
-        fprintf(stderr, "[mcx] pack_ascii: n %lld len0 %u woff[1] %lld woff[n] %lld bound %lld cap_pk %lld rec1 %08x %08x %08x %08x\n", (long long)n, l0, w[0], w[1], (long long)bound, (long long)ctx->cap_pk, p0[0], p0[1], p0[2], p0[3]);
+    if (ctx->have_quals) {
+        TRY(ctx->d_qoff.ensure(ctx, n + 1));
+        CK(cudaMemcpyAsync(ctx->d_qoff, d_offsets, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
     }
-    ctx->n_words = -1;            // not known on the host (and not needed: nothing waits on copy steps)
-    (void)with_quals;
     return MCX_OK;
 }
 
 extern "C" int mcx_push_reads(mcx_ctx *ctx, const uint8_t *bases, const uint8_t *quals, const int64_t *offsets,
                               int64_t n) {
     if (!ctx || !offsets || n < 0 || (n > 0 && !bases)) return fail(ctx, MCX_EINVAL, "mcx_push_reads: bad argument");
-    int rc;
-    if ((rc = begin_push(ctx, "mcx_push_reads", n, quals != nullptr)) != MCX_OK) return rc;
     const int64_t total = n > 0 ? offsets[n] : 0;
-    ctx->n_reads = n; ctx->n_bases = total; ctx->have_quals = quals != nullptr;
-    if ((rc = ensure(ctx, &ctx->d_ascii, &ctx->cap_ascii, total + 16)) != MCX_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_aoffs, &ctx->cap_aoffs, n + 1)) != MCX_OK) return rc;
-    if (quals && (rc = ensure(ctx, &ctx->d_quals, &ctx->cap_quals, total + 32)) != MCX_OK) return rc;
+    TRY(begin_push(ctx, "mcx_push_reads", n, -1, total, quals));
+    TRY(ctx->d_ascii.ensure(ctx, total + 16));
+    TRY(ctx->d_aoffs.ensure(ctx, n + 1));
+    if (quals) TRY(ctx->d_quals.ensure(ctx, total + 32));
     cudaStream_t st = ctx->stream;
-    CK(cudaEventRecord(ctx->ev_h2d0, st));
+    CK(cudaEventRecord(ctx->ev[EV_H2D0], st));
     if (total > 0) CK(cudaMemcpyAsync(ctx->d_ascii, bases, (size_t)total, cudaMemcpyHostToDevice, st));
     if (quals && total > 0) CK(cudaMemcpyAsync(ctx->d_quals, quals, (size_t)total, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(ctx->d_aoffs, offsets, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyHostToDevice, st));
-    CK(cudaEventRecord(ctx->ev[19], st));
+    CK(cudaEventRecord(ctx->ev[EV_H2D1], st));
     ctx->h2d_timed = true;
-    if ((rc = pack_ascii(ctx, ctx->d_ascii, ctx->d_aoffs, n, total, quals != nullptr)) != MCX_OK) return rc;
-    // the qualities keep the caller's offsets (one byte per base, same offsets as the bases)
-    if (quals) {
-        if ((rc = ensure(ctx, &ctx->d_qoff, &ctx->cap_qoff, n + 1)) != MCX_OK) return rc;
-        CK(cudaMemcpyAsync(ctx->d_qoff, ctx->d_aoffs, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyDeviceToDevice, st));
-    }
+    TRY(pack_ascii(ctx, ctx->d_ascii, ctx->d_aoffs, n, total));
     return end_push(ctx);
 }
 
@@ -3001,16 +2997,9 @@ extern "C" int mcx_push_reads_dev(mcx_ctx *ctx, const uint8_t *d_bases, const ui
                                   const int64_t *d_offsets, int64_t n, int64_t total_bytes) {
     if (!ctx || !d_offsets || n < 0 || (n > 0 && !d_bases)) return fail(ctx, MCX_EINVAL, "mcx_push_reads_dev: bad argument");
     if (d_quals && ((uintptr_t)d_quals & 15)) return fail(ctx, MCX_EINVAL, "mcx_push_reads_dev: qualities must be 16-byte aligned");
-    int rc;
-    if ((rc = begin_push(ctx, "mcx_push_reads_dev", n, d_quals != nullptr)) != MCX_OK) return rc;
-    ctx->n_reads = n; ctx->n_bases = total_bytes; ctx->have_quals = d_quals != nullptr;
-    if (!ctx->ext_quals && ctx->d_quals) { CK(cudaFree(ctx->d_quals)); }
-    ctx->d_quals = const_cast<uint8_t *>(d_quals); ctx->ext_quals = true; ctx->cap_quals = 0;
-    if ((rc = pack_ascii(ctx, d_bases, d_offsets, n, total_bytes, d_quals != nullptr)) != MCX_OK) return rc;
-    if (d_quals) {
-        if ((rc = ensure(ctx, &ctx->d_qoff, &ctx->cap_qoff, n + 1)) != MCX_OK) return rc;
-        CK(cudaMemcpyAsync(ctx->d_qoff, d_offsets, (size_t)(n + 1) * sizeof(int64_t), cudaMemcpyDeviceToDevice, ctx->stream));
-    }
+    TRY(begin_push(ctx, "mcx_push_reads_dev", n, -1, total_bytes, d_quals));
+    TRY(ctx->d_quals.borrow(ctx, const_cast<uint8_t *>(d_quals)));
+    TRY(pack_ascii(ctx, d_bases, d_offsets, n, total_bytes));
     return end_push(ctx);
 }
 
@@ -3025,19 +3014,36 @@ extern "C" void mcx_host_free(void *p) { if (p) cudaFreeHost(p); }
 // ------------------------------------------------------------------------------------------------
 // QC
 // ------------------------------------------------------------------------------------------------
+// copy steps that hold packed words [0, words) and quality bytes [0, qbytes) (words < 0: all of them)
+static int steps_holding(const mcx_ctx *ctx, int64_t words, int64_t qbytes) {
+    if (words < 0) return ctx->n_steps;
+    int need = 0;
+    if (words > 0 && ctx->step_words > 0) need = (int)std::min<int64_t>(ctx->n_steps, (words + ctx->step_words - 1) / ctx->step_words);
+    if (ctx->have_quals && qbytes > 0 && ctx->step_qbytes > 0)
+        need = std::max(need, (int)std::min<int64_t>(ctx->n_steps, (qbytes + 15 + ctx->step_qbytes - 1) / ctx->step_qbytes));
+    return need;
+}
 // make the compute stream wait for the copy steps that hold packed words [0, words) and quality bytes [0, qbytes)
 static int wait_copies(mcx_ctx *ctx, int64_t words, int64_t qbytes) {
     if (ctx->steps_waited >= ctx->n_steps) return MCX_OK;
-    int need = 0;
-    if (words < 0) need = ctx->n_steps;
-    else {
-        if (words > 0 && ctx->step_words > 0) need = (int)std::min<int64_t>(ctx->n_steps, (words + ctx->step_words - 1) / ctx->step_words);
-        if (ctx->have_quals && qbytes > 0 && ctx->step_qbytes > 0)
-            need = std::max(need, (int)std::min<int64_t>(ctx->n_steps, (qbytes + 15 + ctx->step_qbytes - 1) / ctx->step_qbytes));
-    }
+    const int need = steps_holding(ctx, words, qbytes);
     for (int k = ctx->steps_waited; k < need; ++k) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_copy[k], 0));
     ctx->steps_waited = std::max(ctx->steps_waited, need);
     return MCX_OK;
+}
+
+static int pushed_on_device(mcx_ctx *ctx, const char *who) {
+    if (!ctx->pushed) return fail(ctx, MCX_ESTATE, std::string(who) + ": no reads pushed");
+    CK(cudaSetDevice(ctx->device));
+    return MCX_OK;
+}
+// have the copy steps that hold packed words [0, words) and quality bytes [0, qbytes) finished? (does not wait)
+static bool copies_arrived(mcx_ctx *ctx, int64_t words, int64_t qbytes) {
+    const int need = steps_holding(ctx, words, qbytes);
+    if (need <= ctx->steps_waited) return true;
+    const cudaError_t q = cudaEventQuery(ctx->ev_copy[need - 1]);   // the steps complete in order
+    if (q != cudaSuccess) (void)cudaGetLastError();                  // cudaErrorNotReady is not an error
+    return q == cudaSuccess;
 }
 
 static void collect_kqc_time(mcx_ctx *ctx);
@@ -3054,73 +3060,79 @@ static int qc_range(mcx_ctx *ctx, int64_t upto) {
     if (upto <= ctx->qc_upto) return MCX_OK;
     const mcx_params &P = ctx->par;
     const int64_t r0 = ctx->qc_upto, nr = upto - r0;
-    CK(cudaEventRecord(ctx->ev[16], ctx->stream));
+    CK(cudaEventRecord(ctx->ev[EV_KQC0], ctx->stream));
     k_qc<<<(unsigned)((nr * 8 + 255) / 256), 256, 0, ctx->stream>>>(read_store(ctx), r0, upto, P.read_length, P.quality_offset,
                                                                   P.min_quality, P.mean_quality, P.max_unknown, ctx->d_code);
-    CK(cudaEventRecord(ctx->ev[17], ctx->stream));
+    CK(cudaEventRecord(ctx->ev[EV_KQC1], ctx->stream));
     ctx->kqc_pending = true;
     ++ctx->launches;
     ctx->qc_upto = upto;
     return MCX_OK;
 }
 
-// after a synchronisation: add the time of the last k_qc launch to ms[10]
+// after a synchronisation: add the time of the last k_qc launch to ms[MS_KQC]
 static void collect_kqc_time(mcx_ctx *ctx) {
     if (!ctx->kqc_pending) return;
-    ctx->ms[10] += elapsed_ms(ctx->ev[16], ctx->ev[17]);
+    ctx->ms[MS_KQC] += elapsed_ms(ctx->ev[EV_KQC0], ctx->ev[EV_KQC1]);
     ctx->kqc_pending = false;
+}
+
+// fingerprints of all pushed reads in d_fp (computed once per push)
+static int ensure_fingerprints(mcx_ctx *ctx) {
+    const int64_t n = ctx->n_reads;
+    TRY(ctx->d_fp.ensure(ctx, std::max<int64_t>(n, 1)));
+    if (n > 0 && !ctx->fp_done) {
+        k_fingerprint<<<(unsigned)((n + 127) / 128), 128, 0, ctx->stream>>>(read_store(ctx), n, ctx->d_fp);
+        ++ctx->launches; ctx->fp_done = true;
+    }
+    return MCX_OK;
 }
 
 // everything decided over all pushed reads: verdicts and, with -d, the duplicates
 static int qc_all(mcx_ctx *ctx) {
     const int64_t n = ctx->n_reads;
     cudaStream_t st = ctx->stream;
-    int rc;
-    if ((rc = wait_copies(ctx, -1, -1)) != MCX_OK) return rc;
-    CK(cudaEventRecord(ctx->ev[14], st));
-    if ((rc = qc_range(ctx, n)) != MCX_OK) return rc;
+    TRY(wait_copies(ctx, -1, -1));
+    CK(cudaEventRecord(ctx->ev[EV_QC0], st));
+    TRY(qc_range(ctx, n));
     if (ctx->par.filter_dups && !ctx->dedup_done && n > 0) {
-        if ((rc = sync_stream(ctx)) != MCX_OK) return rc;          // (k_qc's events are read before they are reused)
-        CK(cudaEventRecord(ctx->ev[18], st));
-        if ((rc = ensure(ctx, &ctx->d_fp, &ctx->cap_fp, n)) != MCX_OK) return rc;
+        TRY(sync_stream(ctx));                             // (k_qc's events are read before they are reused)
+        CK(cudaEventRecord(ctx->ev[EV_DEDUP0], st));
         const int64_t nt = n + ctx->n_store;               // reads of this push + fingerprints kept by earlier pushes
         if (nt >= (1ll << 31)) return fail(ctx, MCX_EINVAL, "mcx: more than 2^31 fingerprints in the duplicate filter");
-        if ((rc = ensure(ctx, &ctx->d_fpa, &ctx->cap_fpa, nt)) != MCX_OK) return rc;
-        if ((rc = ensure(ctx, &ctx->d_fpa2, &ctx->cap_fpa2, nt)) != MCX_OK) return rc;
-        if ((rc = ensure(ctx, &ctx->d_fpi, &ctx->cap_fpi, nt)) != MCX_OK) return rc;
-        if ((rc = ensure(ctx, &ctx->d_fpi2, &ctx->cap_fpi2, nt)) != MCX_OK) return rc;
-        if (!ctx->fp_done) { k_fingerprint<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(read_store(ctx), n, ctx->d_fp); ++ctx->launches; ctx->fp_done = true; }
+        TRY(ctx->d_fpa.ensure(ctx, nt));
+        TRY(ctx->d_fpa2.ensure(ctx, nt));
+        TRY(ctx->d_fpi.ensure(ctx, nt));
+        TRY(ctx->d_fpi2.ensure(ctx, nt));
+        TRY(ensure_fingerprints(ctx));
         if (nt > 1) {
             // one radix sort on the upper 48 bits of the fingerprint brings equal fingerprints together; which read of a
             // group stays is decided by index inside k_mark_dups, so neither a stable sort nor a second key is needed
             const FpStore S{ctx->d_store_a, ctx->d_store_b};
             k_fp_keys<<<(unsigned)((nt + 255) / 256), 256, 0, st>>>(ctx->d_fp, n, S, ctx->n_store, ctx->d_fpa, ctx->d_fpi);
-            size_t tb = 0;
-            CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, ctx->d_fpa, ctx->d_fpa2, ctx->d_fpi, ctx->d_fpi2, (int)nt, 64 - FP_SORT_BITS, 64, st));
-            if ((rc = ensure_temp(ctx, tb)) != MCX_OK) return rc;
-            CK(cub::DeviceRadixSort::SortPairs(ctx->d_temp, tb, ctx->d_fpa, ctx->d_fpa2, ctx->d_fpi, ctx->d_fpi2, (int)nt, 64 - FP_SORT_BITS, 64, st));
+            TRY(cub_run(ctx, "cub::DeviceRadixSort::SortPairs (fingerprints)", [&](void *t, size_t &tb) {
+                return cub::DeviceRadixSort::SortPairs(t, tb, ctx->d_fpa.p, ctx->d_fpa2.p, ctx->d_fpi.p, ctx->d_fpi2.p, (int)nt, 64 - FP_SORT_BITS, 64, st); }));
             k_mark_dups<<<(unsigned)((nt + 255) / 256), 256, 0, st>>>(ctx->d_fpa2, ctx->d_fpi2, ctx->d_fp, S, nt, ctx->d_code);
             ctx->launches += 9;
         }
-        CK(cudaEventRecord(ctx->ev[12], st));
-        if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
-        ctx->ms[11] += elapsed_ms(ctx->ev[18], ctx->ev[12]);
+        CK(cudaEventRecord(ctx->ev[EV_DEDUP1], st));
+        TRY(sync_stream(ctx));
+        ctx->ms[MS_DEDUP] += elapsed_ms(ctx->ev[EV_DEDUP0], ctx->ev[EV_DEDUP1]);
         ctx->dedup_done = true;
     }
-    CK(cudaEventRecord(ctx->ev[15], st));
+    CK(cudaEventRecord(ctx->ev[EV_QC1], st));
     return MCX_OK;
 }
 
 static int qc_counts_all(mcx_ctx *ctx) {
     if (ctx->counts_valid) return MCX_OK;
-    int rc;
-    if ((rc = qc_all(ctx)) != MCX_OK) return rc;
+    TRY(qc_all(ctx));
     const int64_t n = ctx->n_reads;
     cudaStream_t st = ctx->stream;
     CK(cudaMemsetAsync(ctx->d_cnt + C_QCALL, 0, 4 * sizeof(unsigned long long), st));
     if (n > 0) { k_count_codes<<<592, 256, 0, st>>>(ctx->d_code, n, ctx->d_cnt + C_QCALL); ++ctx->launches; }
     CK(cudaMemcpyAsync(ctx->h_cnt + C_QCALL, ctx->d_cnt + C_QCALL, 4 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
+    TRY(sync_stream(ctx));
     const unsigned long long *c = ctx->h_cnt + C_QCALL;
     ctx->qc.n_reads = n; ctx->qc.kept = (int64_t)c[0]; ctx->qc.too_short = (int64_t)c[1];
     ctx->qc.low_qual = (int64_t)c[2]; ctx->qc.dups = (int64_t)c[3];
@@ -3130,20 +3142,17 @@ static int qc_counts_all(mcx_ctx *ctx) {
 
 extern "C" int mcx_qc_export(mcx_ctx *ctx, uint8_t *code, uint64_t *fingerprints) {
     if (!ctx || !code) return fail(ctx, MCX_EINVAL, "mcx_qc_export: null argument");
-    if (!ctx->pushed) return fail(ctx, MCX_ESTATE, "mcx_qc_export: no reads pushed");
-    CK(cudaSetDevice(ctx->device));
+    TRY(pushed_on_device(ctx, "mcx_qc_export"));
     const int64_t n = ctx->n_reads;
     cudaStream_t st = ctx->stream;
     if (n == 0) return MCX_OK;
-    int rc;
-    if ((rc = qc_all(ctx)) != MCX_OK) return rc;
+    TRY(qc_all(ctx));
     CK(cudaMemcpyAsync(code, ctx->d_code, (size_t)n, cudaMemcpyDeviceToHost, st));
     if (fingerprints) {
-        if ((rc = ensure(ctx, &ctx->d_fp, &ctx->cap_fp, n)) != MCX_OK) return rc;
-        if (!ctx->fp_done) { k_fingerprint<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(read_store(ctx), n, ctx->d_fp); ++ctx->launches; ctx->fp_done = true; }
+        TRY(ensure_fingerprints(ctx));
         std::vector<FpKey> h((size_t)n);
         CK(cudaMemcpyAsync(h.data(), ctx->d_fp, (size_t)n * sizeof(FpKey), cudaMemcpyDeviceToHost, st));
-        if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
+        TRY(sync_stream(ctx));
         for (int64_t i = 0; i < n; ++i) { fingerprints[2 * i] = h[(size_t)i].a; fingerprints[2 * i + 1] = h[(size_t)i].b; }
     }
     return sync_stream(ctx);
@@ -3151,10 +3160,8 @@ extern "C" int mcx_qc_export(mcx_ctx *ctx, uint8_t *code, uint64_t *fingerprints
 
 extern "C" int mcx_qc_import(mcx_ctx *ctx, const uint8_t *code) {
     if (!ctx || !code) return fail(ctx, MCX_EINVAL, "mcx_qc_import: null argument");
-    if (!ctx->pushed) return fail(ctx, MCX_ESTATE, "mcx_qc_import: no reads pushed");
-    CK(cudaSetDevice(ctx->device));
-    int rc;
-    if ((rc = qc_all(ctx)) != MCX_OK) return rc;
+    TRY(pushed_on_device(ctx, "mcx_qc_import"));
+    TRY(qc_all(ctx));
     if (ctx->n_reads > 0)
         CK(cudaMemcpyAsync(ctx->d_code, code, (size_t)ctx->n_reads, cudaMemcpyHostToDevice, ctx->stream));
     ctx->counts_valid = false; ctx->searched = false;
@@ -3166,18 +3173,12 @@ extern "C" int mcx_qc_import(mcx_ctx *ctx, const uint8_t *code) {
 // rewrites codes in place and calls mcx_qc_refresh.
 extern "C" int mcx_qc_device(mcx_ctx *ctx, void **d_code, void **d_fingerprints, int64_t *n) {
     if (!ctx || !d_code || !n) return fail(ctx, MCX_EINVAL, "mcx_qc_device: null argument");
-    if (!ctx->pushed) return fail(ctx, MCX_ESTATE, "mcx_qc_device: no reads pushed");
-    CK(cudaSetDevice(ctx->device));
-    int rc;
-    if ((rc = qc_all(ctx)) != MCX_OK) return rc;
+    TRY(pushed_on_device(ctx, "mcx_qc_device"));
+    TRY(qc_all(ctx));
     *n = ctx->n_reads;
     *d_code = ctx->d_code;
     if (d_fingerprints) {
-        if ((rc = ensure(ctx, &ctx->d_fp, &ctx->cap_fp, std::max<int64_t>(ctx->n_reads, 1))) != MCX_OK) return rc;
-        if (ctx->n_reads > 0 && !ctx->fp_done) {
-            k_fingerprint<<<(unsigned)((ctx->n_reads + 127) / 128), 128, 0, ctx->stream>>>(read_store(ctx), ctx->n_reads, ctx->d_fp);
-            ++ctx->launches; ctx->fp_done = true;
-        }
+        TRY(ensure_fingerprints(ctx));
         *d_fingerprints = ctx->d_fp;
     }
     return sync_stream(ctx);
@@ -3185,18 +3186,15 @@ extern "C" int mcx_qc_device(mcx_ctx *ctx, void **d_code, void **d_fingerprints,
 
 extern "C" int mcx_qc_refresh(mcx_ctx *ctx) {
     if (!ctx) return fail(ctx, MCX_EINVAL, "mcx_qc_refresh: null context");
-    if (!ctx->pushed) return fail(ctx, MCX_ESTATE, "mcx_qc_refresh: no reads pushed");
-    CK(cudaSetDevice(ctx->device));
+    TRY(pushed_on_device(ctx, "mcx_qc_refresh"));
     ctx->counts_valid = false; ctx->searched = false;
     return qc_counts_all(ctx);
 }
 
 extern "C" int mcx_qc_counts(mcx_ctx *ctx, mcx_qc *out) {
     if (!ctx || !out) return fail(ctx, MCX_EINVAL, "mcx_qc_counts: null argument");
-    if (!ctx->pushed) return fail(ctx, MCX_ESTATE, "mcx_qc_counts: no reads pushed");
-    CK(cudaSetDevice(ctx->device));
-    int rc;
-    if ((rc = qc_counts_all(ctx)) != MCX_OK) return rc;
+    TRY(pushed_on_device(ctx, "mcx_qc_counts"));
+    TRY(qc_counts_all(ctx));
     *out = ctx->qc;
     return MCX_OK;
 }
@@ -3213,12 +3211,10 @@ extern "C" int mcx_qc_counts(mcx_ctx *ctx, mcx_qc *out) {
 struct XRec { unsigned long long a, b; long long gp; };
 // room for `need` stored fingerprints, keeping the ones there are
 static int reserve_store(mcx_ctx *ctx, int64_t need) {
-    if (need <= ctx->cap_store) return MCX_OK;
+    if (need <= ctx->d_store_a.cap) return MCX_OK;
     const int64_t cap = need + need / 2 + 1024;
-    int rc;
-    if ((rc = grow_keep(ctx, &ctx->d_store_a, ctx->n_store, cap)) != MCX_OK) return rc;
-    if ((rc = grow_keep(ctx, &ctx->d_store_b, ctx->n_store, cap)) != MCX_OK) return rc;
-    ctx->cap_store = cap;
+    TRY(ctx->d_store_a.grow_keep(ctx, ctx->n_store, cap));
+    TRY(ctx->d_store_b.grow_keep(ctx, ctx->n_store, cap));
     return MCX_OK;
 }
 extern "C" int mcx_dedup_reset(mcx_ctx *ctx) {
@@ -3304,33 +3300,30 @@ __global__ void k_x_apply(const uint8_t *__restrict__ marks, const uint32_t *__r
 
 extern "C" int mcx_dedup_begin(mcx_ctx *ctx, int world, int64_t first_index, void **d_send, int64_t *send_counts) {
     if (!ctx || !d_send || !send_counts || world < 1 || world > 64) return fail(ctx, MCX_EINVAL, "mcx_dedup_begin: bad argument (1 <= world <= 64)");
-    if (!ctx->pushed) return fail(ctx, MCX_ESTATE, "mcx_dedup_begin: no reads pushed");
-    CK(cudaSetDevice(ctx->device));
+    TRY(pushed_on_device(ctx, "mcx_dedup_begin"));
     cudaStream_t st = ctx->stream;
     const int64_t n = ctx->n_reads;
-    int rc;
-    if ((rc = qc_all(ctx)) != MCX_OK) return rc;
-    if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
-    CK(cudaEventRecord(ctx->ev[18], st));
-    if ((rc = ensure(ctx, &ctx->d_fp, &ctx->cap_fp, std::max<int64_t>(n, 1))) != MCX_OK) return rc;
-    if (n > 0 && !ctx->fp_done) { k_fingerprint<<<(unsigned)((n + 127) / 128), 128, 0, st>>>(read_store(ctx), n, ctx->d_fp); ++ctx->launches; ctx->fp_done = true; }
-    if ((rc = ensure(ctx, &ctx->d_xsend, &ctx->cap_xsend, std::max<int64_t>(n, 1) * 3)) != MCX_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_fpi, &ctx->cap_fpi, std::max<int64_t>(n, 1))) != MCX_OK) return rc;
+    TRY(qc_all(ctx));
+    TRY(sync_stream(ctx));
+    CK(cudaEventRecord(ctx->ev[EV_DEDUP0], st));
+    TRY(ensure_fingerprints(ctx));
+    TRY(ctx->d_xsend.ensure(ctx, std::max<int64_t>(n, 1) * 3));
+    TRY(ctx->d_fpi.ensure(ctx, std::max<int64_t>(n, 1)));
     unsigned long long *cnt = ctx->d_cnt + C_XCNT, *cur = ctx->d_cnt + C_XCNT + 64 + 0;   // counts, then cursors (exclusive prefix)
     CK(cudaMemsetAsync(cnt, 0, 128 * sizeof(unsigned long long), st));
     if (n > 0) k_x_count<<<592, 256, 0, st>>>(ctx->d_fp, ctx->d_code, n, world, cnt);
     CK(cudaMemcpyAsync(ctx->h_cnt, cnt, 64 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
+    TRY(sync_stream(ctx));
     unsigned long long pre[64], acc = 0;
     for (int o = 0; o < 64; ++o) { pre[o] = acc; if (o < world) { send_counts[o] = (int64_t)ctx->h_cnt[o]; acc += ctx->h_cnt[o]; } }
     ctx->x_nsend = (int64_t)acc;
     CK(cudaMemcpyAsync(cur, pre, 64 * sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
     if (n > 0) k_x_scatter<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(ctx->d_fp, ctx->d_code, n, world, (long long)first_index, cur,
-                                                                       reinterpret_cast<XRec *>(ctx->d_xsend), ctx->d_fpi);
+                                                                       reinterpret_cast<XRec *>(ctx->d_xsend.p), ctx->d_fpi);
     ctx->launches += 2;
-    CK(cudaEventRecord(ctx->ev[12], st));
-    if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
-    ctx->ms[11] += elapsed_ms(ctx->ev[18], ctx->ev[12]);
+    CK(cudaEventRecord(ctx->ev[EV_DEDUP1], st));
+    TRY(sync_stream(ctx));
+    ctx->ms[MS_DEDUP] += elapsed_ms(ctx->ev[EV_DEDUP0], ctx->ev[EV_DEDUP1]);
     *d_send = ctx->d_xsend;
     return MCX_OK;
 }
@@ -3340,50 +3333,42 @@ extern "C" int mcx_dedup_owner(mcx_ctx *ctx, const void *d_recv, int64_t m, void
     if (m >= (1ll << 31)) return fail(ctx, MCX_EINVAL, "mcx_dedup_owner: at most 2^31 records per rank");
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    int rc;
     const int64_t mm = std::max<int64_t>(m, 1);
-    if ((rc = ensure(ctx, &ctx->d_xmarks, &ctx->cap_xmarks, mm)) != MCX_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_fpa, &ctx->cap_fpa, mm)) != MCX_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_fpa2, &ctx->cap_fpa2, mm)) != MCX_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_xkg, &ctx->cap_xkg, mm)) != MCX_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_xvi, &ctx->cap_xvi, mm)) != MCX_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_fpi2, &ctx->cap_fpi2, mm)) != MCX_OK) return rc;
-    CK(cudaEventRecord(ctx->ev[18], st));
-    CK(cudaMemsetAsync(ctx->d_xmarks, 0, (size_t)mm, st));
     const int64_t mt = m + ctx->n_store;                 // the records of this round + the fingerprints this rank has kept before
     if (mt >= (1ll << 31)) return fail(ctx, MCX_EINVAL, "mcx_dedup_owner: more than 2^31 fingerprints on one rank");
+    TRY(ctx->d_xmarks.ensure(ctx, mm));
+    TRY(ctx->d_fpa.ensure(ctx, m > 0 ? mt : 1));
+    TRY(ctx->d_fpa2.ensure(ctx, m > 0 ? mt : 1));
+    TRY(ctx->d_xkg.ensure(ctx, mm));
+    TRY(ctx->d_xvi.ensure(ctx, m > 0 ? mt : 1));
+    TRY(ctx->d_fpi2.ensure(ctx, m > 0 ? mt : 1));
+    CK(cudaEventRecord(ctx->ev[EV_DEDUP0], st));
+    CK(cudaMemsetAsync(ctx->d_xmarks, 0, (size_t)mm, st));
     if (m > 0) {
-        if ((rc = ensure(ctx, &ctx->d_fpa, &ctx->cap_fpa, mt)) != MCX_OK) return rc;
-        if ((rc = ensure(ctx, &ctx->d_fpa2, &ctx->cap_fpa2, mt)) != MCX_OK) return rc;
-        if ((rc = ensure(ctx, &ctx->d_xvi, &ctx->cap_xvi, mt)) != MCX_OK) return rc;
-        if ((rc = ensure(ctx, &ctx->d_fpi2, &ctx->cap_fpi2, mt)) != MCX_OK) return rc;
-        if ((rc = reserve_store(ctx, ctx->n_store + m)) != MCX_OK) return rc;
+        TRY(reserve_store(ctx, ctx->n_store + m));
         const XRec *recv = reinterpret_cast<const XRec *>(d_recv);
         const FpStore S{ctx->d_store_a, ctx->d_store_b};
         k_x_keys<<<(unsigned)((m + 255) / 256), 256, 0, st>>>(recv, m, ctx->d_xkg, ctx->d_fpa, ctx->d_xvi);
         if (ctx->n_store > 0) k_x_keys_store<<<(unsigned)((ctx->n_store + 255) / 256), 256, 0, st>>>(S, m, ctx->n_store, ctx->d_fpa, ctx->d_xvi);
-        size_t tb = 0;
-        CK(cub::DeviceRadixSort::SortPairs(nullptr, tb, ctx->d_fpa, ctx->d_fpa2, ctx->d_xvi, ctx->d_fpi2, (int)mt, 64 - FP_SORT_BITS, 64, st));
-        if ((rc = ensure_temp(ctx, tb)) != MCX_OK) return rc;
-        CK(cub::DeviceRadixSort::SortPairs(ctx->d_temp, tb, ctx->d_fpa, ctx->d_fpa2, ctx->d_xvi, ctx->d_fpi2, (int)mt, 64 - FP_SORT_BITS, 64, st));
+        TRY(cub_run(ctx, "cub::DeviceRadixSort::SortPairs (owned fingerprints)", [&](void *t, size_t &tb) {
+            return cub::DeviceRadixSort::SortPairs(t, tb, ctx->d_fpa.p, ctx->d_fpa2.p, ctx->d_xvi.p, ctx->d_fpi2.p, (int)mt, 64 - FP_SORT_BITS, 64, st); }));
         ctx->h_cnt[C_NSTORE] = (unsigned long long)ctx->n_store;
         CK(cudaMemcpyAsync(ctx->d_cnt + C_NSTORE, ctx->h_cnt + C_NSTORE, sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
         k_x_mark<<<(unsigned)((mt + 255) / 256), 256, 0, st>>>(ctx->d_fpa2, ctx->d_fpi2, recv, S, mt, ctx->d_xmarks, ctx->d_store_a, ctx->d_store_b, ctx->d_cnt + C_NSTORE);
         CK(cudaMemcpyAsync(ctx->h_cnt + C_NSTORE, ctx->d_cnt + C_NSTORE, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
         ctx->launches += 10;
     }
-    CK(cudaEventRecord(ctx->ev[12], st));
-    if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
+    CK(cudaEventRecord(ctx->ev[EV_DEDUP1], st));
+    TRY(sync_stream(ctx));
     if (m > 0) ctx->n_store = (int64_t)ctx->h_cnt[C_NSTORE];
-    ctx->ms[11] += elapsed_ms(ctx->ev[18], ctx->ev[12]);
+    ctx->ms[MS_DEDUP] += elapsed_ms(ctx->ev[EV_DEDUP0], ctx->ev[EV_DEDUP1]);
     *d_marks = ctx->d_xmarks;
     return MCX_OK;
 }
 
 extern "C" int mcx_dedup_finish(mcx_ctx *ctx, const void *d_marks_back) {
     if (!ctx || (ctx->x_nsend > 0 && !d_marks_back)) return fail(ctx, MCX_EINVAL, "mcx_dedup_finish: bad argument");
-    if (!ctx->pushed) return fail(ctx, MCX_ESTATE, "mcx_dedup_finish: no reads pushed");
-    CK(cudaSetDevice(ctx->device));
+    TRY(pushed_on_device(ctx, "mcx_dedup_finish"));
     if (ctx->x_nsend > 0) {
         k_x_apply<<<(unsigned)((ctx->x_nsend + 255) / 256), 256, 0, ctx->stream>>>(reinterpret_cast<const uint8_t *>(d_marks_back), ctx->d_fpi, ctx->x_nsend, ctx->d_code);
         ++ctx->launches;
@@ -3398,31 +3383,40 @@ struct IsKept {
     __device__ __forceinline__ bool operator()(const int32_t &i) const { return code[i] == 0; }
 };
 
-extern "C" int mcx_search(mcx_ctx *ctx, int64_t quota) {
-    if (!ctx) return fail(ctx, MCX_EINVAL, "mcx_search: null context");
-    if (!ctx->pushed) return fail(ctx, MCX_ESTATE, "mcx_search: no reads pushed");
-    CK(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
+struct SearchPlan {
+    int64_t quota, chunk;                      // quota < 0: all kept reads; chunk: reads the frame store and queues are sized for
+    int maxm, fstride, nwr, thr;               // frame length, frame row stride, words of a 12-window mask, report floor
+    uint8_t *frames;
+    bool streaming;                            // rounds of pieces sized by what the host -> device copies have delivered
+    std::vector<int64_t> bounds;               // piece c holds reads [bounds[c], bounds[c + 1])
+    std::vector<long long> bw, bq;             // packed words / quality bytes before bounds[c] (-1: not read back)
+    int pieces() const { return (int)bounds.size() - 1; }
+};
+// sums over the chunks of a search
+struct SearchTally {
+    int64_t sampled = 0, examined = 0;
+    unsigned long long segq = 0, pass = 0, cand = 0, seeds = 0, surv = 0;   // surv: ungapped HSPs of all chunks so far
+    float ms_qc = 0, ms_frames = 0, ms_seg = 0, ms_probe = 0, ms_kprobe = 0, ms_ext = 0, ms_kseed = 0, ms_gap = 0;
+};
+
+// buffer sizes from the chunk size and the MCX_* knobs
+static int plan_search(mcx_ctx *ctx, int64_t quota, SearchPlan &S) {
     const mcx_params &P = ctx->par;
     const int64_t n = ctx->n_reads;
-    int rc;
-    mcx_result &R = ctx->res;
-    memset(&R, 0, sizeof R);
-    unsigned long long *hc = ctx->h_cnt;
-    // buffers
     int64_t per_read = 8;
     if (const char *e = getenv("MCX_SURV_PER_READ")) per_read = std::max(1, atoi(e));
     const int64_t want = std::max<int64_t>((quota >= 0 ? std::min(quota, n) : n) * per_read, 1 << 16);
-    if (ctx->cap_surv < want && (rc = grow_survivors(ctx, 0, want)) != MCX_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_best, &ctx->cap_best, n + 1)) != MCX_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_nrep, &ctx->cap_nrep, n + 1)) != MCX_OK) return rc;
-    if ((rc = ensure(ctx, &ctx->d_bestkey, &ctx->cap_bestkey, n + 1)) != MCX_OK) return rc;
-    const int maxm = (P.read_length + 2) / 3;
+    if (ctx->d_surv.cap < want) TRY(grow_survivors(ctx, 0, want));
+    TRY(ctx->d_best.ensure(ctx, n + 1));
+    TRY(ctx->d_nrep.ensure(ctx, n + 1));
+    TRY(ctx->d_bestkey.ensure(ctx, n + 1));
+    S.quota = quota;
+    S.maxm = (P.read_length + 2) / 3;
     // an ungapped HSP of 49+ can still grow in the gapped stage, so it survives whatever the floor is
-    const int thr = std::max(1, std::min(P.min_report_raw, 49));
+    S.thr = std::max(1, std::min(P.min_report_raw, 49));
     // the stages run per chunk of pushed reads so that the frame store and the queues stay bounded
-    const int fstride = frame_stride(maxm);
-    const int nwr = std::max(1, (maxm - SEG_WINDOW + 1 + 31) / 32);     // words of a 12-window mask
+    S.fstride = frame_stride(S.maxm);
+    S.nwr = std::max(1, (S.maxm - SEG_WINDOW + 1 + 31) / 32);
     int64_t chunk = 2000000, cand_per_read = std::max<int64_t>(96, (int64_t)(0.8 * P.read_length));   // ~0.69 L word-hit postings per read on the marker set
     chunk = std::min<int64_t>(chunk, std::max<int64_t>(250000, 300000000 / P.read_length));   // queues scale with bases, not reads
     if (const char *e = getenv("MCX_CHUNK_READS")) chunk = std::min(2700000, std::max(1, atoi(e)));   // frame rows < 2^24
@@ -3430,312 +3424,273 @@ extern "C" int mcx_search(mcx_ctx *ctx, int64_t quota) {
     int64_t pass_per_read = std::max<int64_t>(32, (int64_t)(0.4 * P.read_length));    // ~0.23 L words per read pass the filter
     if (const char *e = getenv("MCX_PASS_PER_READ")) pass_per_read = std::max(1, atoi(e));
     chunk = std::min<int64_t>(chunk, std::max<int64_t>(n, 1));
-    {
-        const int64_t need_fr = (chunk * 6 + 512) * fstride + 128, need_cand = std::max<int64_t>(chunk * cand_per_read, 1 << 16);
-        const int64_t cap_fr_before = ctx->cap_frames;
-        if ((rc = ensure(ctx, &ctx->d_frames, &ctx->cap_frames, need_fr)) != MCX_OK) return rc;
-        // k_seed reads 16-byte windows around a word without looking at the row ends: whatever lies there must be a residue code
-        if (ctx->cap_frames != cap_fr_before) CK(cudaMemsetAsync(ctx->d_frames, AA_STOP, (size_t)ctx->cap_frames, ctx->stream));
-        if ((rc = ensure(ctx, &ctx->d_cand, &ctx->cap_cand, need_cand)) != MCX_OK) return rc;
-        if ((rc = ensure(ctx, &ctx->d_passq, &ctx->cap_passq, std::max<int64_t>(chunk * pass_per_read, 1 << 16))) != MCX_OK) return rc;
-        if ((rc = ensure(ctx, &ctx->d_seedq, &ctx->cap_seedq, std::max<int64_t>(ctx->cap_cand / 2, 1 << 16))) != MCX_OK) return rc;
-        if ((rc = ensure(ctx, &ctx->d_segq, &ctx->cap_segq, chunk * 6 + 512)) != MCX_OK) return rc;
-        if ((rc = ensure(ctx, &ctx->d_segm, &ctx->cap_segm, (chunk * 6 + 512) * 2 * nwr)) != MCX_OK) return rc;
-        if ((rc = ensure(ctx, &ctx->d_kept, &ctx->cap_kept, chunk + 1)) != MCX_OK) return rc;
-    }
-    uint8_t *const frames = ctx->d_frames + 64;      // rows are also read as aligned words around a position (load_residues)
-    // chunk boundaries; while host -> device copies are in flight the first chunks are small, so that the search starts
-    // as soon as a few tens of megabytes have arrived
-    std::vector<int64_t> bounds(1, 0);
-    // While host -> device copies are in flight the reads are cut into pieces of a sixteenth of a chunk, and every
-    // round of the loop below searches the pieces that have ARRIVED by then (at least two, at most a chunk): with one
-    // GPU on the link that is a small first round and then full chunks; with eight GPUs sharing the host's memory system
-    // (copies 2.3x slower) the rounds stay as large as the link allows and the search never waits for more than it
-    // needs.  (Before: rounds of 1/8, 1/4, 1/2, 1 chunk whatever the link did -- at 8 GPUs the search idled 11 ms of an
-    // 80 ms step waiting for rounds twice as large as what it had just finished.)
-    const bool streaming = ctx->steps_waited < ctx->n_steps && ctx->n_steps > 1 && !P.filter_dups;
-    {
-        const int64_t c = streaming ? std::min<int64_t>(chunk, std::max<int64_t>(chunk / 16, 65536)) : chunk;   // never more than the buffers hold
-        while (bounds.back() < n) bounds.push_back(std::min(n, bounds.back() + c));
-    }
-    const int nb = (int)bounds.size() - 1;
-    std::vector<long long> bw((size_t)nb + 1, -1), bq((size_t)nb + 1, -1);
-    if (ctx->steps_waited < ctx->n_steps && !P.filter_dups) {
-        // where the chunks end in the packed words / quality bytes (the offsets were scanned on the device)
-        for (int c = 1; c <= nb; ++c) {
-            CK(cudaMemcpyAsync(&bw[(size_t)c], ctx->d_woff + bounds[(size_t)c], sizeof(long long), cudaMemcpyDeviceToHost, st));
-            if (ctx->have_quals) CK(cudaMemcpyAsync(&bq[(size_t)c], ctx->d_qoff + bounds[(size_t)c], sizeof(long long), cudaMemcpyDeviceToHost, st));
+    S.chunk = chunk;
+    bool grew = false;
+    TRY(ctx->d_frames.ensure(ctx, (chunk * 6 + 512) * S.fstride + 128, &grew));
+    // k_seed reads 16-byte windows around a word without looking at the row ends: whatever lies there must be a residue code
+    if (grew) CK(cudaMemsetAsync(ctx->d_frames, AA_STOP, (size_t)ctx->d_frames.cap, ctx->stream));
+    TRY(ctx->d_cand.ensure(ctx, std::max<int64_t>(chunk * cand_per_read, 1 << 16)));
+    TRY(ctx->d_passq.ensure(ctx, std::max<int64_t>(chunk * pass_per_read, 1 << 16)));
+    TRY(ctx->d_seedq.ensure(ctx, std::max<int64_t>(ctx->d_cand.cap / 2, 1 << 16)));
+    TRY(ctx->d_segq.ensure(ctx, chunk * 6 + 512));
+    TRY(ctx->d_segm.ensure(ctx, (chunk * 6 + 512) * 2 * S.nwr));
+    TRY(ctx->d_kept.ensure(ctx, chunk + 1));
+    S.frames = ctx->d_frames + 64;             // rows are also read as aligned words around a position (load_residues)
+    return MCX_OK;
+}
+
+// While host -> device copies are in flight the reads are cut into pieces of a sixteenth of a chunk, and every round of
+// the chunk loop searches the pieces that have ARRIVED by then (at least two, at most a chunk): with one GPU on the link
+// that is a small first round and then full chunks; with eight GPUs sharing the host's memory system (copies 2.3x
+// slower) the rounds stay as large as the link allows and the search never waits for more than it needs (fixed rounds of
+// 1/8, 1/4, 1/2, 1 chunk left the search idle 11 ms of an 80 ms step at 8 GPUs).
+static int chunk_bounds(mcx_ctx *ctx, SearchPlan &S) {
+    const int64_t n = ctx->n_reads;
+    S.streaming = ctx->steps_waited < ctx->n_steps && ctx->n_steps > 1 && !ctx->par.filter_dups;
+    const int64_t c = S.streaming ? std::min<int64_t>(S.chunk, std::max<int64_t>(S.chunk / 16, 65536)) : S.chunk;   // never more than the buffers hold
+    S.bounds.assign(1, 0);
+    while (S.bounds.back() < n) S.bounds.push_back(std::min(n, S.bounds.back() + c));
+    const int nb = S.pieces();
+    S.bw.assign((size_t)nb + 1, -1); S.bq.assign((size_t)nb + 1, -1);
+    if (ctx->steps_waited < ctx->n_steps && !ctx->par.filter_dups) {
+        // where the pieces end in the packed words / quality bytes (the offsets were scanned on the device)
+        for (int k = 1; k <= nb; ++k) {
+            CK(cudaMemcpyAsync(&S.bw[(size_t)k], ctx->d_woff + S.bounds[(size_t)k], sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
+            if (ctx->have_quals) CK(cudaMemcpyAsync(&S.bq[(size_t)k], ctx->d_qoff + S.bounds[(size_t)k], sizeof(long long), cudaMemcpyDeviceToHost, ctx->stream));
         }
-        if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
-        if (nb > 0 && (bw[(size_t)nb] != ctx->n_words || (ctx->have_quals && bq[(size_t)nb] != ctx->n_bases)))
+        TRY(sync_stream(ctx));
+        if (nb > 0 && (S.bw[(size_t)nb] != ctx->n_words || (ctx->have_quals && S.bq[(size_t)nb] != ctx->n_bases)))
             return fail(ctx, MCX_EINVAL, "mcx_search: the pushed lengths do not add up to the pushed words / bases");
     }
-    CK(cudaMemsetAsync(ctx->d_nrep, 0, (size_t)(n + 1) * sizeof(int32_t), st));
-    CK(cudaMemsetAsync(ctx->d_bestkey, 0, (size_t)(n + 1) * sizeof(unsigned long long), st));
-    CK(cudaMemsetAsync(ctx->d_cnt, 0, 4 * sizeof(unsigned long long), st));
-    CK(cudaMemsetAsync(ctx->d_cnt + C_SURV, 0, (C_N - C_SURV) * sizeof(unsigned long long), st));
-    CK(cudaMemsetAsync(ctx->d_acc, 0, (3 + 2 * MCX_N_FAM) * sizeof(unsigned long long), st));
-    CK(cudaMemsetAsync(ctx->d_abl, 0, (size_t)MCX_N_FAM * MCX_LEN_BINS * sizeof(unsigned long long), st));
-    if (n > 0) { k_fill_i32<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(ctx->d_best, n, -1); ++ctx->launches; }
-    float ms_qc = 0;
-    if (P.filter_dups || ctx->counts_valid) {     // -d is decided over all reads before anything is searched
-        if ((rc = qc_all(ctx)) != MCX_OK) return rc;
-        if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
-        ms_qc += elapsed_ms(ctx->ev[14], ctx->ev[15]);
-    }
+    return MCX_OK;
+}
 
-    float ms_frames = 0, ms_seg = 0, ms_probe = 0, ms_ext = 0, ms_gap = 0, ms_kprobe = 0, ms_kseed = 0;
-    unsigned long long n_surv = 0, n_cand_total = 0, n_seeds_total = 0, n_pass_total = 0, n_segq_total = 0;
-    int64_t remaining = quota, sampled = 0, examined = 0;
-    auto arrived = [&](long long words, long long qbytes) -> bool {     // have the copy steps holding [0, words) / [0, qbytes) finished?
-        int need = 0;
-        if (words > 0 && ctx->step_words > 0) need = (int)std::min<int64_t>(ctx->n_steps, (words + ctx->step_words - 1) / ctx->step_words);
-        if (ctx->have_quals && qbytes > 0 && ctx->step_qbytes > 0)
-            need = std::max(need, (int)std::min<int64_t>(ctx->n_steps, (qbytes + 15 + ctx->step_qbytes - 1) / ctx->step_qbytes));
-        if (need <= ctx->steps_waited) return true;
-        const cudaError_t q = cudaEventQuery(ctx->ev_copy[need - 1]);   // the steps complete in order
-        if (q != cudaSuccess) (void)cudaGetLastError();                  // cudaErrorNotReady is not an error
-        return q == cudaSuccess;
+// K1 on the reads of pieces [c, c1): verdicts, the list of kept reads, the -n cut and the verdict counts up to the read
+// that fills it (mc.py:356 leaves the loop there); nr = kept reads searched, -1: all of them, counted on the device
+static int qc_chunk(mcx_ctx *ctx, const SearchPlan &S, int c, int c1, SearchTally &T, int64_t &nr) {
+    cudaStream_t st = ctx->stream;
+    unsigned long long *hc = ctx->h_cnt;
+    const int64_t r0 = S.bounds[(size_t)c], r1 = S.bounds[(size_t)c1];
+    TRY(wait_copies(ctx, S.bw[(size_t)c1], S.bq[(size_t)c1]));
+    CK(cudaEventRecord(ctx->ev[EV_QC0], st));
+    TRY(qc_range(ctx, r1));
+    thrust::counting_iterator<int32_t> it((int32_t)r0);
+    TRY(cub_run(ctx, "cub::DeviceSelect::If (kept reads)", [&](void *t, size_t &tb) {
+        return cub::DeviceSelect::If(t, tb, it, ctx->d_kept.p, ctx->d_cnt + C_NKEPT, (int)(r1 - r0), IsKept{ctx->d_code}, st); }));
+    ctx->launches += 2;
+    int64_t upto = r1;                         // verdicts counted up to here
+    nr = -1;
+    if (S.quota >= 0) {
+        CK(cudaMemcpyAsync(hc + C_NKEPT, ctx->d_cnt + C_NKEPT, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        TRY(sync_stream(ctx));
+        const int64_t kept_c = (int64_t)hc[C_NKEPT], remaining = S.quota - T.sampled;
+        nr = std::min(kept_c, remaining);
+        if (nr == remaining && nr > 0) {     // the quota is filled inside this chunk: by its nr-th kept read
+            int32_t cut = 0;
+            CK(cudaMemcpyAsync(&cut, ctx->d_kept + (nr - 1), sizeof cut, cudaMemcpyDeviceToHost, st));
+            TRY(sync_stream(ctx));
+            upto = (int64_t)cut + 1;
+        }
+        if (nr < kept_c) { hc[C_NKEPT + 1] = (unsigned long long)nr; CK(cudaMemcpyAsync(ctx->d_cnt + C_NKEPT, hc + C_NKEPT + 1, sizeof(unsigned long long), cudaMemcpyHostToDevice, st)); }
+    }
+    if (upto > r0) { k_count_codes<<<592, 256, 0, st>>>(ctx->d_code + r0, upto - r0, ctx->d_cnt + C_QC0); ++ctx->launches; }
+    T.examined = upto;
+    return MCX_OK;
+}
+
+// six frames of every searched read, then the full SEG of the frames k_frames queued (resident blocks, queue length read
+// on the device); nr_max bounds the launches
+static int frames_and_seg(mcx_ctx *ctx, const SearchPlan &S, int64_t nr_max) {
+    cudaStream_t st = ctx->stream;
+    const int L = ctx->par.read_length;
+    CK(cudaMemsetAsync(ctx->d_cnt + C_SEGQ, 0, 2 * sizeof(unsigned long long), st));   // SEG queue length, k_seg's work counter
+    CK(cudaEventRecord(ctx->ev[EV_FRAMES0], st));
+    constexpr int NTF = MCX_FRAMES_NT;         // a multiple of 6: whole reads per block
+    FrameArgs F;
+    F.S = read_store(ctx); F.kept = ctx->d_kept; F.first = 0; F.n_search = ctx->d_cnt + C_NKEPT;
+    F.L = L; F.frames = S.frames; F.segq = ctx->d_segq; F.n_segq = ctx->d_cnt + C_SEGQ;
+    F.segm = ctx->d_segm; F.nwr = S.nwr;
+    const size_t fsmem = sizeof(SegTab) + 256 + (size_t)S.fstride * NTF + (size_t)((NTF / 6 * L + 3) & ~3) + (size_t)2 * S.nwr * NTF * 4;
+    CK(cudaFuncSetAttribute(k_frames<NTF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)fsmem));
+    k_frames<NTF><<<(unsigned)((nr_max * 6 + NTF - 1) / NTF), NTF, fsmem, st>>>(F, S.fstride);
+    ++ctx->launches;
+    CK(cudaEventRecord(ctx->ev[EV_SEG0], st));
+    constexpr int SW = MCX_SEG_W;
+    const size_t smem = 2 * SEG_TAB * sizeof(double) + sizeof(SegTab) + 128 + SEG_TRI + (size_t)SW * seg_warp_bytes(S.fstride, S.maxm);
+    CK(cudaFuncSetAttribute(k_seg<SW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    unsigned resident = 0;
+    TRY(resident_blocks(ctx, k_seg<SW>, SW * 32, smem, resident));
+    k_seg<SW><<<(unsigned)std::min<unsigned long long>((nr_max * 6 + SW - 1) / SW, resident), SW * 32, smem, st>>>(
+        S.frames, S.fstride, L, ctx->d_segq, ctx->d_segm, S.nwr, ctx->d_cnt + C_SEGQ, S.maxm, reinterpret_cast<unsigned int *>(ctx->d_cnt + C_WORK));
+    ++ctx->launches;
+    CK(cudaEventRecord(ctx->ev[EV_PROBE0], st));
+    return MCX_OK;
+}
+
+// K2: probe -> resolve -> seed -> walk, queue lengths read on the device, one read-back behind them; a queue that
+// overflowed is sized for what was seen and the chunk's seed stage runs again
+static int seed_stage(mcx_ctx *ctx, const SearchPlan &S, int64_t nr_max, SearchTally &T) {
+    cudaStream_t st = ctx->stream;
+    unsigned long long *hc = ctx->h_cnt;
+    const unsigned long long surv_before = T.surv;
+    unsigned long long n_cand = 0, n_seeds = 0, n_pass = 0;
+    constexpr int NTP = MCX_PROBE_NT, NTR = MCX_RESOLVE_NT;
+    const size_t psmem = (size_t)S.fstride * NTP;
+    unsigned res_probe = 0, res_resolve = 0, res_seed = 0, res_walk = 0;
+    CK(cudaFuncSetAttribute(k_probe<NTP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)psmem));
+    TRY(resident_blocks(ctx, k_probe<NTP>, NTP, psmem, res_probe));
+    TRY(resident_blocks(ctx, k_resolve<NTR>, NTR, 0, res_resolve));
+    TRY(resident_blocks(ctx, k_seed<SEED_NT>, SEED_NT, 0, res_seed));
+    TRY(resident_blocks(ctx, k_walk<WALK_NT>, WALK_NT, 0, res_walk));
+    auto row_blocks = [](unsigned resident, int nt, unsigned long long cap) -> unsigned {   // resident blocks per sub-queue row
+        const unsigned long long want = ((unsigned long long)resident * 2 + NQ - 1) / NQ;
+        return (unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>(want, (cap + nt - 1) / nt));
     };
-    for (int c = 0, c1 = 0; c < nb && (quota < 0 || remaining > 0); c = c1) {
-        c1 = c + 1;
-        if (streaming)                           // a second piece whatever has arrived (if a chunk holds two), then what has arrived
-            while (c1 < nb && bounds[(size_t)c1 + 1] - bounds[(size_t)c] <= chunk &&
-                   (c1 - c < 2 || arrived(bw[(size_t)c1 + 1], bq[(size_t)c1 + 1]))) ++c1;
-        const int64_t r0 = bounds[(size_t)c], r1 = bounds[(size_t)c1], nr_in = r1 - r0;
-        // ---- K1 on this chunk: verdicts, list of kept reads
-        if ((rc = wait_copies(ctx, bw[(size_t)c1], bq[(size_t)c1])) != MCX_OK) return rc;
-        CK(cudaEventRecord(ctx->ev[14], st));
-        if ((rc = qc_range(ctx, r1)) != MCX_OK) return rc;
-        {
-            size_t tb = 0;
-            thrust::counting_iterator<int32_t> it((int32_t)r0);
-            CK(cub::DeviceSelect::If(nullptr, tb, it, ctx->d_kept, ctx->d_cnt + C_NKEPT, (int)nr_in, IsKept{ctx->d_code}, st));
-            if ((rc = ensure_temp(ctx, tb)) != MCX_OK) return rc;
-            CK(cub::DeviceSelect::If(ctx->d_temp, tb, it, ctx->d_kept, ctx->d_cnt + C_NKEPT, (int)nr_in, IsKept{ctx->d_code}, st));
-            ctx->launches += 2;
-        }
-        int64_t upto = r1;                      // verdicts counted up to here (mc.py:356 leaves the loop at the read that fills -n)
-        int64_t nr = -1;                        // kept reads of the chunk that are searched; -1: all of them, count on the device
-        if (quota >= 0) {
-            CK(cudaMemcpyAsync(hc + C_NKEPT, ctx->d_cnt + C_NKEPT, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-            if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
-            const int64_t kept_c = (int64_t)hc[C_NKEPT];
-            nr = std::min(kept_c, remaining);
-            if (nr == remaining && nr > 0) {    // the quota is filled inside this chunk: by its nr-th kept read
-                int32_t cut = 0;
-                CK(cudaMemcpyAsync(&cut, ctx->d_kept + (nr - 1), sizeof cut, cudaMemcpyDeviceToHost, st));
-                if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
-                upto = (int64_t)cut + 1;
-            }
-            if (nr < kept_c) { hc[C_NKEPT + 1] = (unsigned long long)nr; CK(cudaMemcpyAsync(ctx->d_cnt + C_NKEPT, hc + C_NKEPT + 1, sizeof(unsigned long long), cudaMemcpyHostToDevice, st)); }
-            remaining -= nr;
-        }
-        if (upto > r0) { k_count_codes<<<592, 256, 0, st>>>(ctx->d_code + r0, upto - r0, ctx->d_cnt + C_QC0); ++ctx->launches; }
-        examined = upto;
-        if (nr == 0) continue;
-        const int64_t nr_max = nr < 0 ? nr_in : nr;        // launch bound; the kernels read the count on the device
-        CK(cudaMemsetAsync(ctx->d_cnt + C_SEGQ, 0, 2 * sizeof(unsigned long long), st));   // SEG queue length, k_seg's work counter
-        CK(cudaEventRecord(ctx->ev[2], st));
-        constexpr int NTF = MCX_FRAMES_NT;      // a multiple of 6: whole reads per block
-        {
-            FrameArgs F;
-            F.S = read_store(ctx); F.kept = ctx->d_kept; F.first = 0; F.n_search = ctx->d_cnt + C_NKEPT;
-            F.L = P.read_length; F.frames = frames; F.segq = ctx->d_segq; F.n_segq = ctx->d_cnt + C_SEGQ;
-            F.segm = ctx->d_segm; F.nwr = nwr;
-            const size_t smem = sizeof(SegTab) + 256 + (size_t)fstride * NTF + (size_t)((NTF / 6 * P.read_length + 3) & ~3) + (size_t)2 * nwr * NTF * 4;
-            CK(cudaFuncSetAttribute(k_frames<NTF>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            k_frames<NTF><<<(unsigned)((nr_max * 6 + NTF - 1) / NTF), NTF, smem, st>>>(F, fstride);
-            ++ctx->launches;
-        }
-        CK(cudaEventRecord(ctx->ev[10], st));
-        {   // full SEG of the queued frames: resident blocks, queue length read on the device
-            constexpr int SW = MCX_SEG_W;
-            const size_t smem = 2 * SEG_TAB * sizeof(double) + sizeof(SegTab) + 128 + SEG_TRI + (size_t)SW * seg_warp_bytes(fstride, maxm);
-            CK(cudaFuncSetAttribute(k_seg<SW>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            int per_sm = 0;
-            CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_seg<SW>, SW * 32, smem));
-            const unsigned long long resident = (unsigned long long)std::max(per_sm, 1) * (unsigned long long)ctx->n_sm;
-            k_seg<SW><<<(unsigned)std::min<unsigned long long>((nr_max * 6 + SW - 1) / SW, resident), SW * 32, smem, st>>>(
-                frames, fstride, P.read_length, ctx->d_segq, ctx->d_segm, nwr, ctx->d_cnt + C_SEGQ, maxm, reinterpret_cast<unsigned int *>(ctx->d_cnt + C_WORK));
-            ++ctx->launches;
-        }
-        CK(cudaEventRecord(ctx->ev[11], st));
-        const unsigned long long surv_before = n_surv;
-        unsigned long long n_cand = 0, n_seeds = 0, n_pass = 0;
-        for (int attempt = 0;; ++attempt) {
-            // ---- K2: probe -> seed -> walk, queue lengths read on the device; one read-back behind the three
-            CK(cudaMemsetAsync(ctx->d_qcnt, 0, 2 * NQ * sizeof(unsigned long long), st));
-            CK(cudaMemsetAsync(ctx->d_cnt + C_SEEDQ, 0, sizeof(unsigned long long), st));
-            ProbeArgs A;
-            A.n_reads = ctx->d_cnt + C_NKEPT; A.L = P.read_length; A.db = ctx->db; A.frames = frames; A.cand = ctx->d_cand;
-            A.n_cand = ctx->d_qcnt; A.cap_cand = (unsigned long long)(ctx->cap_cand / NQ);
-            A.passq = ctx->d_passq; A.n_pass = ctx->d_qcnt + NQ; A.cap_pass = (unsigned long long)(ctx->cap_passq / NQ);
-            constexpr int NTP = MCX_PROBE_NT, NTR = MCX_RESOLVE_NT;
-            const size_t smem = (size_t)fstride * NTP;
-            CK(cudaFuncSetAttribute(k_probe<NTP>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            {
-                int per_sm = 0;
-                if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_probe<NTP>, NTP, smem) != cudaSuccess || per_sm < 1) per_sm = 1;
-                const unsigned long long resident = (unsigned long long)per_sm * ctx->n_sm;
-                k_probe<NTP><<<(unsigned)std::min<unsigned long long>((nr_max * 6 + NTP - 1) / NTP, resident), NTP, smem, st>>>(A, fstride);
-            }
-            if (attempt == 0) CK(cudaEventRecord(ctx->ev[20], st));
-            auto row_blocks = [&](auto kernel, int nt, unsigned long long cap) -> unsigned {   // resident blocks per sub-queue row
-                int per_sm = 0;
-                if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, nt, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
-                const unsigned long long want = ((unsigned long long)per_sm * ctx->n_sm * 2 + NQ - 1) / NQ;
-                return (unsigned)std::max<unsigned long long>(1, std::min<unsigned long long>(want, (cap + nt - 1) / nt));
-            };
-            k_resolve<NTR><<<dim3(row_blocks(k_resolve<NTR>, NTR, A.cap_pass), NQ), NTR, 0, st>>>(A);
-            ++ctx->launches;
-            if (attempt == 0) CK(cudaEventRecord(ctx->ev[3], st));
-            ExtArgs E;
-            E.kept = ctx->d_kept; E.first = 0; E.L = P.read_length; E.fstride = fstride; E.thr_report = thr; E.db = ctx->db;
-            E.frames = frames; E.cand = ctx->d_cand; E.qfill = ctx->d_qcnt;
-            E.cap_cand = (unsigned long long)(ctx->cap_cand / NQ);
-            E.surv = ctx->d_surv; E.cap_surv = (unsigned long long)ctx->cap_surv;
-            E.n_surv = ctx->d_cnt + C_SURV; E.n_seedq = ctx->d_cnt + C_SEEDQ;
-            E.seedq = ctx->d_seedq; E.cap_seedq = (unsigned long long)ctx->cap_seedq;
-            {   // duplicate filter: at least two slots per survivor the list can take
-                int bits = 16;
-                while ((1ll << bits) < 2 * ctx->cap_surv) ++bits;
-                if ((rc = ensure(ctx, &ctx->d_seen, &ctx->cap_seen, 1ll << bits)) != MCX_OK) return rc;
-                CK(cudaMemsetAsync(ctx->d_seen, 0xff, (size_t)(1ll << bits) * sizeof(unsigned long long), st));
-                E.seen = ctx->d_seen; E.seen_mask = (1ull << bits) - 1; E.seen_shift = 64 - bits;
-            }
-            k_seed<SEED_NT><<<dim3(row_blocks(k_seed<SEED_NT>, SEED_NT, E.cap_cand), NQ), SEED_NT, 0, st>>>(E);
-            if (attempt == 0) CK(cudaEventRecord(ctx->ev[21], st));
-            {
-                int per_sm = 0;
-                if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_walk<WALK_NT>, WALK_NT, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
-                k_walk<WALK_NT><<<(unsigned)(per_sm * ctx->n_sm * 8), WALK_NT, 0, st>>>(E);
-            }
-            ctx->launches += 3;
-            CK(cudaEventRecord(ctx->ev[8], st));
-            CK(cudaMemcpyAsync(hc + C_N, ctx->d_qcnt, 2 * NQ * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-            CK(cudaMemcpyAsync(hc, ctx->d_cnt, C_N * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-            if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
-            unsigned long long worst = 0, worst_pass = 0;
-            n_cand = 0;
-            for (int q = 0; q < NQ; ++q) { n_cand += hc[C_N + q]; worst = std::max(worst, hc[C_N + q]); worst_pass = std::max(worst_pass, hc[C_N + NQ + q]); n_pass += hc[C_N + NQ + q]; }
-            n_seeds = hc[C_SEEDQ];
-            const bool over_pass = (int64_t)worst_pass > ctx->cap_passq / NQ;
-            const bool over_cand = (int64_t)worst > ctx->cap_cand / NQ, over_seed = (int64_t)n_seeds > ctx->cap_seedq,
-                       over_surv = (int64_t)hc[C_SURV] > ctx->cap_surv;
-            if (!over_pass && !over_cand && !over_seed && !over_surv) { n_surv = hc[C_SURV]; break; }
-            if (attempt >= 4) return fail(ctx, MCX_ENOMEM, "mcx_search: a queue (filter passes / candidates / seeds / survivors) overflowed after regrowth");
-            // the fills are exact (of what the earlier queues let through): size the queue that overflowed for what was
-            // seen and run the chunk's seed stage again
-            n_pass = 0;
-            if (over_pass && (rc = ensure(ctx, &ctx->d_passq, &ctx->cap_passq, (int64_t)(worst_pass + worst_pass / 16 + 1024) * NQ)) != MCX_OK) return rc;
-            if (over_cand && (rc = ensure(ctx, &ctx->d_cand, &ctx->cap_cand, (int64_t)(worst + worst / 16 + 1024) * NQ)) != MCX_OK) return rc;
-            if ((over_cand || over_seed) && (rc = ensure(ctx, &ctx->d_seedq, &ctx->cap_seedq, std::max<int64_t>((int64_t)(n_seeds + n_seeds / 8), ctx->cap_cand / 2))) != MCX_OK) return rc;
-            if (over_surv && (rc = grow_survivors(ctx, (int64_t)surv_before, (int64_t)hc[C_SURV] + (int64_t)hc[C_SURV] / 4)) != MCX_OK) return rc;
-            hc[C_SURV] = surv_before;
-            CK(cudaMemcpyAsync(ctx->d_cnt + C_SURV, hc + C_SURV, sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
-        }
-        n_cand_total += n_cand; n_seeds_total += n_seeds; n_pass_total += n_pass; n_segq_total += hc[C_SEGQ];
-        sampled += nr < 0 ? (int64_t)hc[C_NKEPT] : nr;
-        if (n_surv > surv_before) {
-            GapArgs G;
-            G.L = P.read_length; G.fstride = fstride; G.db = ctx->db; G.frames = frames; G.surv = ctx->d_surv;
-            G.first = (int64_t)surv_before; G.n_surv = (int64_t)(n_surv - surv_before);
-            G.hsp = ctx->d_hsp; G.keys = ctx->d_keys; G.idx = ctx->d_idx; G.counters = ctx->d_cnt + C_GAPPED;
-            if ((rc = ensure(ctx, &ctx->d_gitems, &ctx->cap_gitems, 6 * G.n_surv)) != MCX_OK) return rc;
-            if ((rc = ensure(ctx, &ctx->d_gext, &ctx->cap_gext, 2 * G.n_surv)) != MCX_OK) return rc;
-            G.items = ctx->d_gitems; G.ext = ctx->d_gext; G.n_items = ctx->d_cnt + C_ITEMS; G.n_items_total = ctx->d_cnt + C_NGAPTOT;
-            CK(cudaMemsetAsync(ctx->d_gext, 0, (size_t)(2 * G.n_surv) * sizeof(GExtRec), st));
-            CK(cudaMemsetAsync(ctx->d_cnt + C_ITEMS, 0, sizeof(unsigned long long), st));
-            // work list (padded with all-ones keys up to its bound, so that it can be sorted without knowing its
-            // length on the host) -> sorted by remaining query length -> screening pass -> complete pass for the
-            // extensions that gain -> (never seen: wide-window fallback) ; no host round trip in between
-            unsigned long long *list1 = ctx->d_gitems + G.n_surv * 2, *gainers = ctx->d_gitems + G.n_surv * 4, *wide = ctx->d_gitems;
-            CK(cudaMemsetAsync(G.items, 0xff, (size_t)(2 * G.n_surv) * sizeof(unsigned long long), st));
-            k_gap_list<<<(unsigned)((G.n_surv + 255) / 256), 256, 0, st>>>(G);
-            {
-                size_t tb = 0;
-                CK(cub::DeviceRadixSort::SortKeys(nullptr, tb, G.items, list1, (int)(2 * G.n_surv), 32, 40, st));
-                if ((rc = ensure_temp(ctx, tb)) != MCX_OK) return rc;
-                CK(cub::DeviceRadixSort::SortKeys(ctx->d_temp, tb, G.items, list1, (int)(2 * G.n_surv), 32, 40, st));
-            }
-            CK(cudaMemsetAsync(ctx->d_cnt + C_ITEMS2, 0, sizeof(unsigned long long), st));
-            CK(cudaMemsetAsync(ctx->d_cnt + C_WORK1, 0, 2 * sizeof(unsigned long long), st));
-            CK(cudaMemsetAsync(ctx->d_cnt + C_NWIDE, 0, 3 * sizeof(unsigned long long), st));
-            auto resident = [&](auto kernel, int nt, unsigned want) -> unsigned {      // blocks of a grid that is resident at once
-                int per_sm = 0;
-                if (cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kernel, nt, 0) != cudaSuccess || per_sm < 1) per_sm = 1;
-                return std::max(1u, std::min(want, (unsigned)(per_sm * ctx->n_sm)));
-            };
-            constexpr int SNT = MCX_SCR_NT, FNT = MCX_FULL_NT;
-            const unsigned bound = (unsigned)(2 * G.n_surv);
-            k_gap_screen<SNT><<<resident(k_gap_screen<SNT>, SNT, (bound + SNT - 1) / SNT), SNT, 0, st>>>(G, list1, gainers, ctx->d_cnt + C_ITEMS2);
-            CK(cudaMemcpyAsync(hc + C_ITEMS2, ctx->d_cnt + C_ITEMS2, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-            if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
-            const int64_t n_gain = (int64_t)hc[C_ITEMS2];
-            // complete DP + traceback of the extensions that gain, in batches that bound the direction scratch
-            const int rows_per_ext = maxm;
-            const int64_t per_ext = (int64_t)rows_per_ext * DIR_ROW_WORDS;
-            int64_t batch = std::max<int64_t>(1, (int64_t)(2ll << 30) / (per_ext * 4));       // 2 GB of directions at most
-            if (const char *e = getenv("MCX_GAP_BATCH")) batch = std::max(1, atoi(e));
-            batch = std::min(batch, std::max<int64_t>(n_gain, 1));
-            if (n_gain > 0 && (rc = ensure(ctx, &ctx->d_dirs, &ctx->cap_dirs, batch * per_ext)) != MCX_OK) return rc;
-            for (int64_t g0 = 0; g0 < n_gain; g0 += batch) {
-                const int64_t ng = std::min(batch, n_gain - g0);
-                CK(cudaMemsetAsync(ctx->d_cnt + C_WORK1, 0, sizeof(unsigned long long), st));
-                k_gap_dp<FNT><<<resident(k_gap_dp<FNT>, FNT, (unsigned)((ng + FNT - 1) / FNT)), FNT, 0, st>>>(
-                    G, gainers, g0, ng, ctx->d_dirs, rows_per_ext, wide, ctx->d_cnt + C_NWIDE, reinterpret_cast<unsigned int *>(ctx->d_cnt + C_WORK1));
-                k_gap_trace<<<(unsigned)((ng + 127) / 128), 128, 0, st>>>(G, gainers, g0, ng, ctx->d_dirs, rows_per_ext);
-                ctx->launches += 2;
-            }
-            {   // fallback for extensions whose window outgrew the ring: score pass + statistics pass with rows in local memory
-                unsigned long long *wide2 = ctx->d_gitems + G.n_surv;
-                unsigned int *work2 = reinterpret_cast<unsigned int *>(ctx->d_cnt + C_WORK2), *work3 = reinterpret_cast<unsigned int *>(ctx->d_cnt + C_NWIDE + 2);
-                constexpr int GW = MAX_FRAME + GAP_SLACK + 2;
-                k_gap_dir<GAP_NT, GW, false><<<resident(k_gap_dir<GAP_NT, GW, false>, GAP_NT, 64), GAP_NT, 0, st>>>(G, wide, ctx->d_cnt + C_NWIDE, wide2, ctx->d_cnt + C_NWIDE + 1, work2);
-                k_gap_dir<GAP_NT, GW, true><<<resident(k_gap_dir<GAP_NT, GW, true>, GAP_NT, 64), GAP_NT, 0, st>>>(G, wide2, ctx->d_cnt + C_NWIDE + 1, nullptr, nullptr, work3);
-            }
-            ctx->launches += 8;
-            k_gap_finish<<<(unsigned)((G.n_surv + 255) / 256), 256, 0, st>>>(G);
-            ctx->launches += 3;
-        }
-        CK(cudaEventRecord(ctx->ev[9], st));
-        if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
-        ms_qc += elapsed_ms(ctx->ev[14], ctx->ev[2]);
-        ms_frames += elapsed_ms(ctx->ev[2], ctx->ev[10]);
-        ms_seg += elapsed_ms(ctx->ev[10], ctx->ev[11]);
-        ms_probe += elapsed_ms(ctx->ev[11], ctx->ev[3]);
-        ms_kprobe += elapsed_ms(ctx->ev[11], ctx->ev[20]);
-        ms_kseed += elapsed_ms(ctx->ev[3], ctx->ev[21]);
-        ms_ext += elapsed_ms(ctx->ev[3], ctx->ev[8]);
-        ms_gap += elapsed_ms(ctx->ev[8], ctx->ev[9]);
-    }
-    if (P.filter_dups && ctx->fp_done && examined > 0) {
-        // streamed -d: the reads kept by this push are what later pushes of the run must not repeat (mc.py:355)
-        if ((rc = reserve_store(ctx, ctx->n_store + examined)) != MCX_OK) return rc;
-        hc[C_NSTORE] = (unsigned long long)ctx->n_store;
-        CK(cudaMemcpyAsync(ctx->d_cnt + C_NSTORE, hc + C_NSTORE, sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
-        k_store_append<<<(unsigned)((examined + 255) / 256), 256, 0, st>>>(ctx->d_fp, ctx->d_code, examined, ctx->d_store_a, ctx->d_store_b, ctx->d_cnt + C_NSTORE);
+    for (int attempt = 0;; ++attempt) {
+        CK(cudaMemsetAsync(ctx->d_qcnt, 0, 2 * NQ * sizeof(unsigned long long), st));
+        CK(cudaMemsetAsync(ctx->d_cnt + C_SEEDQ, 0, sizeof(unsigned long long), st));
+        ProbeArgs A;
+        A.n_reads = ctx->d_cnt + C_NKEPT; A.L = ctx->par.read_length; A.db = ctx->db; A.frames = S.frames; A.cand = ctx->d_cand;
+        A.n_cand = ctx->d_qcnt; A.cap_cand = (unsigned long long)(ctx->d_cand.cap / NQ);
+        A.passq = ctx->d_passq; A.n_pass = ctx->d_qcnt + NQ; A.cap_pass = (unsigned long long)(ctx->d_passq.cap / NQ);
+        k_probe<NTP><<<(unsigned)std::min<unsigned long long>((nr_max * 6 + NTP - 1) / NTP, res_probe), NTP, psmem, st>>>(A, S.fstride);
+        if (attempt == 0) CK(cudaEventRecord(ctx->ev[EV_KPROBE1], st));
+        k_resolve<NTR><<<dim3(row_blocks(res_resolve, NTR, A.cap_pass), NQ), NTR, 0, st>>>(A);
         ++ctx->launches;
+        if (attempt == 0) CK(cudaEventRecord(ctx->ev[EV_SEED0], st));
+        ExtArgs E;
+        E.kept = ctx->d_kept; E.first = 0; E.L = ctx->par.read_length; E.fstride = S.fstride; E.thr_report = S.thr; E.db = ctx->db;
+        E.frames = S.frames; E.cand = ctx->d_cand; E.qfill = ctx->d_qcnt;
+        E.cap_cand = (unsigned long long)(ctx->d_cand.cap / NQ);
+        E.surv = ctx->d_surv; E.cap_surv = (unsigned long long)ctx->d_surv.cap;
+        E.n_surv = ctx->d_cnt + C_SURV; E.n_seedq = ctx->d_cnt + C_SEEDQ;
+        E.seedq = ctx->d_seedq; E.cap_seedq = (unsigned long long)ctx->d_seedq.cap;
+        {   // duplicate filter: at least two slots per survivor the list can take
+            int bits = 16;
+            while ((1ll << bits) < 2 * ctx->d_surv.cap) ++bits;
+            TRY(ctx->d_seen.ensure(ctx, 1ll << bits));
+            CK(cudaMemsetAsync(ctx->d_seen, 0xff, (size_t)(1ll << bits) * sizeof(unsigned long long), st));
+            E.seen = ctx->d_seen; E.seen_mask = (1ull << bits) - 1; E.seen_shift = 64 - bits;
+        }
+        k_seed<SEED_NT><<<dim3(row_blocks(res_seed, SEED_NT, E.cap_cand), NQ), SEED_NT, 0, st>>>(E);
+        if (attempt == 0) CK(cudaEventRecord(ctx->ev[EV_KSEED1], st));
+        k_walk<WALK_NT><<<res_walk * 8, WALK_NT, 0, st>>>(E);
+        ctx->launches += 3;
+        CK(cudaEventRecord(ctx->ev[EV_GAP0], st));
+        CK(cudaMemcpyAsync(hc + C_N, ctx->d_qcnt, 2 * NQ * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        CK(cudaMemcpyAsync(hc, ctx->d_cnt, C_N * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+        TRY(sync_stream(ctx));
+        unsigned long long worst = 0, worst_pass = 0;
+        n_cand = 0;
+        for (int q = 0; q < NQ; ++q) { n_cand += hc[C_N + q]; worst = std::max(worst, hc[C_N + q]); worst_pass = std::max(worst_pass, hc[C_N + NQ + q]); n_pass += hc[C_N + NQ + q]; }
+        n_seeds = hc[C_SEEDQ];
+        const bool over_pass = (int64_t)worst_pass > ctx->d_passq.cap / NQ;
+        const bool over_cand = (int64_t)worst > ctx->d_cand.cap / NQ, over_seed = (int64_t)n_seeds > ctx->d_seedq.cap,
+                   over_surv = (int64_t)hc[C_SURV] > ctx->d_surv.cap;
+        if (!over_pass && !over_cand && !over_seed && !over_surv) { T.surv = hc[C_SURV]; break; }
+        if (attempt >= 4) return fail(ctx, MCX_ENOMEM, "mcx_search: a queue (filter passes / candidates / seeds / survivors) overflowed after regrowth");
+        // the fills are exact (of what the earlier queues let through): size the queue that overflowed for what was seen
+        n_pass = 0;
+        if (over_pass) TRY(ctx->d_passq.ensure(ctx, (int64_t)(worst_pass + worst_pass / 16 + 1024) * NQ));
+        if (over_cand) TRY(ctx->d_cand.ensure(ctx, (int64_t)(worst + worst / 16 + 1024) * NQ));
+        if (over_cand || over_seed) TRY(ctx->d_seedq.ensure(ctx, std::max<int64_t>((int64_t)(n_seeds + n_seeds / 8), ctx->d_cand.cap / 2)));
+        if (over_surv) TRY(grow_survivors(ctx, (int64_t)surv_before, (int64_t)hc[C_SURV] + (int64_t)hc[C_SURV] / 4));
+        hc[C_SURV] = surv_before;
+        CK(cudaMemcpyAsync(ctx->d_cnt + C_SURV, hc + C_SURV, sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
     }
-    R.sampled_reads = sampled;
-    R.n_seed_hits = (int64_t)n_surv;
-    ctx->n_cand_last = (int64_t)n_cand_total;
-    ctx->work[0] = (int64_t)n_segq_total; ctx->work[1] = (int64_t)n_pass_total; ctx->work[2] = (int64_t)n_cand_total;
-    ctx->work[3] = (int64_t)n_seeds_total; ctx->work[4] = (int64_t)n_surv;
-    const int64_t ns = (int64_t)n_surv;
-    CK(cudaEventRecord(ctx->ev[4], st));
+    T.cand += n_cand; T.seeds += n_seeds; T.pass += n_pass; T.segq += hc[C_SEGQ];
+    return MCX_OK;
+}
+
+// gapped extension of the survivors [first, first + count): work list (padded with all-ones keys up to its bound, so that
+// it can be sorted without knowing its length on the host) -> sorted by remaining query length -> screening pass ->
+// complete DP + traceback for the extensions that gain -> (never seen: wide-window fallback) -> finish
+static int gapped_stage(mcx_ctx *ctx, const SearchPlan &S, int64_t first, int64_t count) {
+    cudaStream_t st = ctx->stream;
+    GapArgs G;
+    G.L = ctx->par.read_length; G.fstride = S.fstride; G.db = ctx->db; G.frames = S.frames; G.surv = ctx->d_surv;
+    G.first = first; G.n_surv = count;
+    G.hsp = ctx->d_hsp; G.keys = ctx->d_keys; G.idx = ctx->d_idx; G.counters = ctx->d_cnt + C_GAPPED;
+    TRY(ctx->d_gitems.ensure(ctx, 6 * G.n_surv));
+    TRY(ctx->d_gext.ensure(ctx, 2 * G.n_surv));
+    G.items = ctx->d_gitems; G.ext = ctx->d_gext; G.n_items = ctx->d_cnt + C_ITEMS; G.n_items_total = ctx->d_cnt + C_NGAPTOT;
+    CK(cudaMemsetAsync(ctx->d_gext, 0, (size_t)(2 * G.n_surv) * sizeof(GExtRec), st));
+    CK(cudaMemsetAsync(ctx->d_cnt + C_ITEMS, 0, sizeof(unsigned long long), st));
+    unsigned long long *list1 = ctx->d_gitems + G.n_surv * 2, *gainers = ctx->d_gitems + G.n_surv * 4, *wide = ctx->d_gitems;
+    CK(cudaMemsetAsync(G.items, 0xff, (size_t)(2 * G.n_surv) * sizeof(unsigned long long), st));
+    k_gap_list<<<(unsigned)((G.n_surv + 255) / 256), 256, 0, st>>>(G);
+    TRY(cub_run(ctx, "cub::DeviceRadixSort::SortKeys (gapped work list)", [&](void *t, size_t &tb) {
+        return cub::DeviceRadixSort::SortKeys(t, tb, G.items, list1, (int)(2 * G.n_surv), 32, 40, st); }));
+    CK(cudaMemsetAsync(ctx->d_cnt + C_ITEMS2, 0, sizeof(unsigned long long), st));
+    CK(cudaMemsetAsync(ctx->d_cnt + C_WORK1, 0, 2 * sizeof(unsigned long long), st));
+    CK(cudaMemsetAsync(ctx->d_cnt + C_NWIDE, 0, 3 * sizeof(unsigned long long), st));
+    constexpr int SNT = MCX_SCR_NT, FNT = MCX_FULL_NT, GW = MAX_FRAME + GAP_SLACK + 2;
+    unsigned res_screen = 0, res_dp = 0, res_dir = 0, res_dir2 = 0;
+    TRY(resident_blocks(ctx, k_gap_screen<SNT>, SNT, 0, res_screen));
+    TRY(resident_blocks(ctx, k_gap_dp<FNT>, FNT, 0, res_dp));
+    TRY(resident_blocks(ctx, k_gap_dir<GAP_NT, GW, false>, GAP_NT, 0, res_dir));
+    TRY(resident_blocks(ctx, k_gap_dir<GAP_NT, GW, true>, GAP_NT, 0, res_dir2));
+    auto grid = [](unsigned want, unsigned resident) { return std::max(1u, std::min(want, resident)); };
+    k_gap_screen<SNT><<<grid(((unsigned)(2 * G.n_surv) + SNT - 1) / SNT, res_screen), SNT, 0, st>>>(G, list1, gainers, ctx->d_cnt + C_ITEMS2);
+    CK(cudaMemcpyAsync(ctx->h_cnt + C_ITEMS2, ctx->d_cnt + C_ITEMS2, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    TRY(sync_stream(ctx));
+    const int64_t n_gain = (int64_t)ctx->h_cnt[C_ITEMS2];
+    // complete DP + traceback of the extensions that gain, in batches that bound the direction scratch
+    const int rows_per_ext = S.maxm;
+    const int64_t per_ext = (int64_t)rows_per_ext * DIR_ROW_WORDS;
+    int64_t batch = std::max<int64_t>(1, (int64_t)(2ll << 30) / (per_ext * 4));       // 2 GB of directions at most
+    if (const char *e = getenv("MCX_GAP_BATCH")) batch = std::max(1, atoi(e));
+    batch = std::min(batch, std::max<int64_t>(n_gain, 1));
+    if (n_gain > 0) TRY(ctx->d_dirs.ensure(ctx, batch * per_ext));
+    for (int64_t g0 = 0; g0 < n_gain; g0 += batch) {
+        const int64_t ng = std::min(batch, n_gain - g0);
+        CK(cudaMemsetAsync(ctx->d_cnt + C_WORK1, 0, sizeof(unsigned long long), st));
+        k_gap_dp<FNT><<<grid((unsigned)((ng + FNT - 1) / FNT), res_dp), FNT, 0, st>>>(
+            G, gainers, g0, ng, ctx->d_dirs, rows_per_ext, wide, ctx->d_cnt + C_NWIDE, reinterpret_cast<unsigned int *>(ctx->d_cnt + C_WORK1));
+        k_gap_trace<<<(unsigned)((ng + 127) / 128), 128, 0, st>>>(G, gainers, g0, ng, ctx->d_dirs, rows_per_ext);
+        ctx->launches += 2;
+    }
+    // fallback for extensions whose window outgrew the ring: score pass + statistics pass with rows in local memory
+    unsigned long long *wide2 = ctx->d_gitems + G.n_surv;
+    unsigned int *work2 = reinterpret_cast<unsigned int *>(ctx->d_cnt + C_WORK2), *work3 = reinterpret_cast<unsigned int *>(ctx->d_cnt + C_NWIDE + 2);
+    k_gap_dir<GAP_NT, GW, false><<<grid(64, res_dir), GAP_NT, 0, st>>>(G, wide, ctx->d_cnt + C_NWIDE, wide2, ctx->d_cnt + C_NWIDE + 1, work2);
+    k_gap_dir<GAP_NT, GW, true><<<grid(64, res_dir2), GAP_NT, 0, st>>>(G, wide2, ctx->d_cnt + C_NWIDE + 1, nullptr, nullptr, work3);
+    ctx->launches += 8;
+    k_gap_finish<<<(unsigned)((G.n_surv + 255) / 256), 256, 0, st>>>(G);
+    ctx->launches += 3;
+    return MCX_OK;
+}
+
+// streamed -d: the reads kept by this push are what later pushes of the run must not repeat (mc.py:355)
+static int append_kept_fingerprints(mcx_ctx *ctx, int64_t examined) {
+    TRY(reserve_store(ctx, ctx->n_store + examined));
+    ctx->h_cnt[C_NSTORE] = (unsigned long long)ctx->n_store;
+    CK(cudaMemcpyAsync(ctx->d_cnt + C_NSTORE, ctx->h_cnt + C_NSTORE, sizeof(unsigned long long), cudaMemcpyHostToDevice, ctx->stream));
+    k_store_append<<<(unsigned)((examined + 255) / 256), 256, 0, ctx->stream>>>(ctx->d_fp, ctx->d_code, examined, ctx->d_store_a, ctx->d_store_b, ctx->d_cnt + C_NSTORE);
+    ++ctx->launches;
+    return MCX_OK;
+}
+
+// sort the ungapped HSPs of all chunks, classify, read the sums back and fill mcx_result, the counters and the timings
+static int classify_and_collect(mcx_ctx *ctx, const SearchTally &T, bool stored) {
+    cudaStream_t st = ctx->stream;
+    unsigned long long *hc = ctx->h_cnt;
+    mcx_result &R = ctx->res;
+    R.sampled_reads = T.sampled;
+    R.n_seed_hits = (int64_t)T.surv;
+    ctx->work[0] = (int64_t)T.segq; ctx->work[1] = (int64_t)T.pass; ctx->work[2] = (int64_t)T.cand;
+    ctx->work[3] = (int64_t)T.seeds; ctx->work[4] = (int64_t)T.surv;
+    const int64_t ns = (int64_t)T.surv;
+    CK(cudaEventRecord(ctx->ev[EV_SORT0], st));
     if (ns > 0) {
-        size_t tb = 0;
-        CK(cub::DeviceMergeSort::SortPairs(nullptr, tb, ctx->d_keys, ctx->d_idx, ns, SortKeyLess(), st));
-        if ((rc = ensure_temp(ctx, tb)) != MCX_OK) return rc;
-        CK(cub::DeviceMergeSort::SortPairs(ctx->d_temp, tb, ctx->d_keys, ctx->d_idx, ns, SortKeyLess(), st));
+        TRY(cub_run(ctx, "cub::DeviceMergeSort::SortPairs (HSPs)", [&](void *t, size_t &tb) {
+            return cub::DeviceMergeSort::SortPairs(t, tb, ctx->d_keys.p, ctx->d_idx.p, ns, SortKeyLess(), st); }));
         ctx->launches += 3;
     }
-    CK(cudaEventRecord(ctx->ev[5], st));
+    CK(cudaEventRecord(ctx->ev[EV_CLS0], st));
     if (ns > 0) {
         ClsArgs C;
-        C.keys = ctx->d_keys; C.n = ns; C.L = P.read_length; C.min_report = P.min_report_raw;
+        C.keys = ctx->d_keys; C.n = ns; C.L = ctx->par.read_length; C.min_report = ctx->par.min_report_raw;
         C.db = ctx->db; C.keep = ctx->d_keep; C.nrep = ctx->d_nrep; C.bestkey = ctx->d_bestkey;
         C.best_subject = ctx->d_best; C.acc = ctx->d_acc; C.aln_by_len = ctx->d_abl;
         C.caplist = ctx->d_hflag; C.n_cap = ctx->d_cnt + C_NCAP;
@@ -3747,30 +3702,84 @@ extern "C" int mcx_search(mcx_ctx *ctx, int64_t quota) {
         k_cls_sum<<<cb, 256, 0, st>>>(C);
         ctx->launches += 5;
     }
-    CK(cudaEventRecord(ctx->ev[6], st));
+    CK(cudaEventRecord(ctx->ev[EV_D2H0], st));
     std::vector<unsigned long long> acc(3 + 2 * MCX_N_FAM), abl((size_t)MCX_N_FAM * MCX_LEN_BINS);
     CK(cudaMemcpyAsync(acc.data(), ctx->d_acc, acc.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(abl.data(), ctx->d_abl, abl.size() * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     CK(cudaMemcpyAsync(hc, ctx->d_cnt, C_N * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
-    CK(cudaEventRecord(ctx->ev[7], st));
-    if ((rc = sync_stream(ctx)) != MCX_OK) return rc;
+    CK(cudaEventRecord(ctx->ev[EV_D2H1], st));
+    TRY(sync_stream(ctx));
     R.too_short = (int64_t)hc[C_QC0 + 1]; R.low_qual = (int64_t)hc[C_QC0 + 2]; R.dups = (int64_t)hc[C_QC0 + 3];
-    if (P.filter_dups && ctx->fp_done && examined > 0) ctx->n_store = (int64_t)hc[C_NSTORE];
+    if (stored) ctx->n_store = (int64_t)hc[C_NSTORE];
     R.reads_with_hits = (int64_t)acc[0]; R.reads_classified = (int64_t)acc[1]; R.n_hsp = (int64_t)acc[2];
     R.n_gapped = (int64_t)hc[C_NGAPTOT]; R.gapped_cells = (int64_t)hc[C_CELLS];
     R.n_capped_reads = (int64_t)hc[C_NCAP];
     if (getenv("MCX_DEBUG")) fprintf(stderr, "[mcx] filter passes %llu, candidates %llu, accepted seeds %llu, ungapped HSPs %llu; gapped extensions %llu, with gain > 0: %llu, cells %llu; host syncs %lld\n",
-                                     n_pass_total, n_cand_total, n_seeds_total, n_surv, hc[C_NGAPTOT], hc[C_GAPPED], hc[C_CELLS], (long long)ctx->host_syncs);
+                                     T.pass, T.cand, T.seeds, T.surv, hc[C_NGAPTOT], hc[C_GAPPED], hc[C_CELLS], (long long)ctx->host_syncs);
     for (int f = 0; f < MCX_N_FAM; ++f) { R.fam_hits[f] = (int64_t)acc[3 + f]; R.fam_aln[f] = (int64_t)acc[3 + MCX_N_FAM + f]; }
     for (size_t k = 0; k < abl.size(); ++k) R.aln_by_len[k] = (int64_t)abl[k];
-    ctx->ms_detail[0] = ms_kprobe; ctx->ms_detail[1] = ms_probe - ms_kprobe; ctx->ms_detail[2] = ms_kseed; ctx->ms_detail[3] = ms_ext - ms_kseed;
-    ctx->ms[1] = ms_qc; ctx->ms[2] = ms_probe; ctx->ms[7] = ms_ext; ctx->ms[3] = ms_gap; ctx->ms[8] = ms_frames; ctx->ms[9] = ms_seg;
-    ctx->ms[4] = elapsed_ms(ctx->ev[4], ctx->ev[5]);
-    ctx->ms[5] = elapsed_ms(ctx->ev[5], ctx->ev[6]);
-    ctx->ms[6] = elapsed_ms(ctx->ev[6], ctx->ev[7]);
-    if (ctx->h2d_timed && cudaEventQuery(ctx->ev[19]) == cudaSuccess) ctx->ms[0] = elapsed_ms(ctx->ev_h2d0, ctx->ev[19]);
+    ctx->ms_detail[MSD_KPROBE] = T.ms_kprobe; ctx->ms_detail[MSD_KRESOLVE] = T.ms_probe - T.ms_kprobe;
+    ctx->ms_detail[MSD_KSEED] = T.ms_kseed; ctx->ms_detail[MSD_KWALK] = T.ms_ext - T.ms_kseed;
+    ctx->ms[MS_QC] = T.ms_qc; ctx->ms[MS_PROBE] = T.ms_probe; ctx->ms[MS_EXTEND] = T.ms_ext; ctx->ms[MS_GAPPED] = T.ms_gap;
+    ctx->ms[MS_FRAMES] = T.ms_frames; ctx->ms[MS_SEG] = T.ms_seg;
+    ctx->ms[MS_SORT] = elapsed_ms(ctx->ev[EV_SORT0], ctx->ev[EV_CLS0]);
+    ctx->ms[MS_CLASSIFY] = elapsed_ms(ctx->ev[EV_CLS0], ctx->ev[EV_D2H0]);
+    ctx->ms[MS_D2H] = elapsed_ms(ctx->ev[EV_D2H0], ctx->ev[EV_D2H1]);
+    if (ctx->h2d_timed && cudaEventQuery(ctx->ev[EV_H2D1]) == cudaSuccess) ctx->ms[MS_H2D] = elapsed_ms(ctx->ev[EV_H2D0], ctx->ev[EV_H2D1]);
     (void)cudaGetLastError();
-    ctx->n_hsp_sorted = ns;
+    return MCX_OK;
+}
+
+extern "C" int mcx_search(mcx_ctx *ctx, int64_t quota) {
+    if (!ctx) return fail(ctx, MCX_EINVAL, "mcx_search: null context");
+    TRY(pushed_on_device(ctx, "mcx_search"));
+    cudaStream_t st = ctx->stream;
+    const int64_t n = ctx->n_reads;
+    memset(&ctx->res, 0, sizeof ctx->res);
+    SearchPlan S;
+    TRY(plan_search(ctx, quota, S));
+    TRY(chunk_bounds(ctx, S));
+    CK(cudaMemsetAsync(ctx->d_nrep, 0, (size_t)(n + 1) * sizeof(int32_t), st));
+    CK(cudaMemsetAsync(ctx->d_bestkey, 0, (size_t)(n + 1) * sizeof(unsigned long long), st));
+    CK(cudaMemsetAsync(ctx->d_cnt, 0, 4 * sizeof(unsigned long long), st));
+    CK(cudaMemsetAsync(ctx->d_cnt + C_SURV, 0, (C_N - C_SURV) * sizeof(unsigned long long), st));
+    CK(cudaMemsetAsync(ctx->d_acc, 0, (3 + 2 * MCX_N_FAM) * sizeof(unsigned long long), st));
+    CK(cudaMemsetAsync(ctx->d_abl, 0, (size_t)MCX_N_FAM * MCX_LEN_BINS * sizeof(unsigned long long), st));
+    if (n > 0) { k_fill_i32<<<(unsigned)((n + 255) / 256), 256, 0, st>>>(ctx->d_best, n, -1); ++ctx->launches; }
+    SearchTally T;
+    if (ctx->par.filter_dups || ctx->counts_valid) {     // -d is decided over all reads before anything is searched
+        TRY(qc_all(ctx));
+        TRY(sync_stream(ctx));
+        T.ms_qc += elapsed_ms(ctx->ev[EV_QC0], ctx->ev[EV_QC1]);
+    }
+    for (int c = 0, c1 = 0; c < S.pieces() && (quota < 0 || T.sampled < quota); c = c1) {
+        c1 = c + 1;
+        if (S.streaming)                       // a second piece whatever has arrived (if a chunk holds two), then what has arrived
+            while (c1 < S.pieces() && S.bounds[(size_t)c1 + 1] - S.bounds[(size_t)c] <= S.chunk &&
+                   (c1 - c < 2 || copies_arrived(ctx, S.bw[(size_t)c1 + 1], S.bq[(size_t)c1 + 1]))) ++c1;
+        int64_t nr = 0;
+        TRY(qc_chunk(ctx, S, c, c1, T, nr));
+        if (nr == 0) continue;
+        const int64_t nr_max = nr < 0 ? S.bounds[(size_t)c1] - S.bounds[(size_t)c] : nr;   // launch bound; the kernels read the count on the device
+        TRY(frames_and_seg(ctx, S, nr_max));
+        const unsigned long long surv_before = T.surv;
+        TRY(seed_stage(ctx, S, nr_max, T));
+        T.sampled += nr < 0 ? (int64_t)ctx->h_cnt[C_NKEPT] : nr;
+        if (T.surv > surv_before) TRY(gapped_stage(ctx, S, (int64_t)surv_before, (int64_t)(T.surv - surv_before)));
+        CK(cudaEventRecord(ctx->ev[EV_GAP1], st));
+        TRY(sync_stream(ctx));
+        T.ms_qc += elapsed_ms(ctx->ev[EV_QC0], ctx->ev[EV_FRAMES0]);
+        T.ms_frames += elapsed_ms(ctx->ev[EV_FRAMES0], ctx->ev[EV_SEG0]);
+        T.ms_seg += elapsed_ms(ctx->ev[EV_SEG0], ctx->ev[EV_PROBE0]);
+        T.ms_probe += elapsed_ms(ctx->ev[EV_PROBE0], ctx->ev[EV_SEED0]);
+        T.ms_kprobe += elapsed_ms(ctx->ev[EV_PROBE0], ctx->ev[EV_KPROBE1]);
+        T.ms_kseed += elapsed_ms(ctx->ev[EV_SEED0], ctx->ev[EV_KSEED1]);
+        T.ms_ext += elapsed_ms(ctx->ev[EV_SEED0], ctx->ev[EV_GAP0]);
+        T.ms_gap += elapsed_ms(ctx->ev[EV_GAP0], ctx->ev[EV_GAP1]);
+    }
+    const bool stored = ctx->par.filter_dups && ctx->fp_done && T.examined > 0;
+    if (stored) TRY(append_kept_fingerprints(ctx, T.examined));
+    TRY(classify_and_collect(ctx, T, stored));
     ctx->searched = true;
     return MCX_OK;
 }
@@ -3787,16 +3796,13 @@ extern "C" int mcx_get_hits(mcx_ctx *ctx, mcx_hit *out, int64_t cap, int64_t *n)
     if (!ctx->searched) return fail(ctx, MCX_ESTATE, "mcx_get_hits: no search has run");
     CK(cudaSetDevice(ctx->device));
     *n = ctx->res.n_hsp;
-    const int64_t ns = ctx->n_hsp_sorted;
+    const int64_t ns = ctx->res.n_seed_hits;              // the HSPs sorted by the search
     if (!out || cap <= 0 || ns == 0) return MCX_OK;
     cudaStream_t st = ctx->stream;
-    int rc;
     k_keep_sorted<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(ctx->d_keep, ns, ctx->d_hflag);
     CK(cudaMemsetAsync(ctx->d_hflag + ns, 0, sizeof(int32_t), st));
-    size_t tb = 0;
-    CK(cub::DeviceScan::ExclusiveSum(nullptr, tb, ctx->d_hflag, ctx->d_hpos, (int)(ns + 1), st));
-    if ((rc = ensure_temp(ctx, tb)) != MCX_OK) return rc;
-    CK(cub::DeviceScan::ExclusiveSum(ctx->d_temp, tb, ctx->d_hflag, ctx->d_hpos, (int)(ns + 1), st));
+    TRY(cub_run(ctx, "cub::DeviceScan::ExclusiveSum (reported HSPs)", [&](void *t, size_t &tb) {
+        return cub::DeviceScan::ExclusiveSum(t, tb, ctx->d_hflag.p, ctx->d_hpos.p, (int)(ns + 1), st); }));
     k_gather_hits<<<(unsigned)((ns + 255) / 256), 256, 0, st>>>(ctx->d_hsp, ctx->d_idx, ctx->d_keep, ctx->d_hpos, ns, ctx->d_hits_out);
     const int64_t take = std::min<int64_t>(cap, ctx->res.n_hsp);
     CK(cudaMemcpyAsync(out, ctx->d_hits_out, (size_t)take * sizeof(mcx_hit), cudaMemcpyDeviceToHost, st));
@@ -3837,28 +3843,32 @@ __global__ void __launch_bounds__(256) k_dpx_bench(int iters, int seed, int *out
     if (r == 0x7fffffff) out[0] = r;                      // keeps the chains alive
 }
 
-extern "C" int mcx_dpx_peak(mcx_ctx *ctx, double *gops_per_s) {
-    if (!ctx || !gops_per_s) return fail(ctx, MCX_EINVAL, "mcx_dpx_peak: null argument");
-    CK(cudaSetDevice(ctx->device));
+// best rate of reps 1..3 of a microbenchmark launch: `work` units over its device time, in 1e9 per second
+template <typename F>
+static int bench_rate(mcx_ctx *ctx, double work, F launch, double *rate) {
     cudaStream_t st = ctx->stream;
-    int sms = 0;
-    CK(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, ctx->device));
-    const int blocks = sms * 8, iters = 1 << 14;
-    int *d_out = reinterpret_cast<int *>(ctx->d_cnt);     // never written in practice
     double best = 0.0;
     for (int rep = 0; rep < 4; ++rep) {
-        CK(cudaEventRecord(ctx->ev[12], st));
-        k_dpx_bench<<<blocks, 256, 0, st>>>(iters, 12345 + rep, d_out);
-        CK(cudaEventRecord(ctx->ev[13], st));
+        CK(cudaEventRecord(ctx->ev[EV_BENCH0], st));
+        launch(rep);
+        CK(cudaEventRecord(ctx->ev[EV_BENCH1], st));
         CK(cudaStreamSynchronize(st));
         CK(cudaGetLastError());
         float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, ctx->ev[12], ctx->ev[13]));
-        const double ops = (double)blocks * 256.0 * (double)iters * 16.0;    // DPX thread-instructions
-        if (rep > 0) best = std::max(best, ops / (ms * 1e-3) / 1e9);
+        CK(cudaEventElapsedTime(&ms, ctx->ev[EV_BENCH0], ctx->ev[EV_BENCH1]));
+        if (rep > 0) best = std::max(best, work / (ms * 1e-3) / 1e9);
     }
-    *gops_per_s = best;
+    *rate = best;
     return MCX_OK;
+}
+
+extern "C" int mcx_dpx_peak(mcx_ctx *ctx, double *gops_per_s) {
+    if (!ctx || !gops_per_s) return fail(ctx, MCX_EINVAL, "mcx_dpx_peak: null argument");
+    CK(cudaSetDevice(ctx->device));
+    const int blocks = ctx->n_sm * 8, iters = 1 << 14;
+    int *d_out = reinterpret_cast<int *>(ctx->d_cnt.p);   // never written in practice
+    const double ops = (double)blocks * 256.0 * (double)iters * 16.0;    // DPX thread-instructions
+    return bench_rate(ctx, ops, [&](int rep) { k_dpx_bench<<<blocks, 256, 0, ctx->stream>>>(iters, 12345 + rep, d_out); }, gops_per_s);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -3882,40 +3892,29 @@ __global__ void __launch_bounds__(256) k_l2_bench(const uint32_t *__restrict__ w
 extern "C" int mcx_l2_peak(mcx_ctx *ctx, double *gsectors_per_s) {
     if (!ctx || !gsectors_per_s) return fail(ctx, MCX_EINVAL, "mcx_l2_peak: null argument");
     CK(cudaSetDevice(ctx->device));
-    cudaStream_t st = ctx->stream;
     const int blocks = ctx->n_sm * 8, iters = 512;
     uint32_t *d_out = reinterpret_cast<uint32_t *>(ctx->d_cnt + C_N - 1);
-    double best = 0.0;
-    for (int rep = 0; rep < 4; ++rep) {
-        CK(cudaEventRecord(ctx->ev[12], st));
-        k_l2_bench<<<blocks, 256, 0, st>>>(reinterpret_cast<const uint32_t *>(ctx->db.filt_a), (4u << FILT_BITS) - 1u, iters, 777u + rep, d_out);
-        CK(cudaEventRecord(ctx->ev[13], st));
-        CK(cudaStreamSynchronize(st));
-        CK(cudaGetLastError());
-        float ms = 0.f;
-        CK(cudaEventElapsedTime(&ms, ctx->ev[12], ctx->ev[13]));
-        const double loads = (double)blocks * 256.0 * (double)iters * 8.0;
-        if (rep > 0) best = std::max(best, loads / (ms * 1e-3) / 1e9);
-    }
-    *gsectors_per_s = best;
-    return MCX_OK;
+    const double loads = (double)blocks * 256.0 * (double)iters * 8.0;
+    return bench_rate(ctx, loads, [&](int rep) {
+        k_l2_bench<<<blocks, 256, 0, ctx->stream>>>(reinterpret_cast<const uint32_t *>(ctx->db.filt_a), (4u << FILT_BITS) - 1u, iters, 777u + rep, d_out);
+    }, gsectors_per_s);
 }
 
 extern "C" int mcx_search_counters(mcx_ctx *ctx, int64_t out[8]) {
     if (!ctx || !out) return fail(ctx, MCX_EINVAL, "mcx_search_counters: null argument");
-    memcpy(out, ctx->work, sizeof(int64_t) * 8);
+    memcpy(out, ctx->work, sizeof ctx->work);
     return MCX_OK;
 }
 
 extern "C" int mcx_timings_detail(mcx_ctx *ctx, float ms[4]) {
     if (!ctx || !ms) return fail(ctx, MCX_EINVAL, "mcx_timings_detail: null argument");
-    memcpy(ms, ctx->ms_detail, sizeof(float) * 4);
+    memcpy(ms, ctx->ms_detail, sizeof ctx->ms_detail);
     return MCX_OK;
 }
 
 extern "C" int mcx_timings(mcx_ctx *ctx, float ms[12], int64_t *launches) {
     if (!ctx || !ms) return fail(ctx, MCX_EINVAL, "mcx_timings: null argument");
-    memcpy(ms, ctx->ms, sizeof(float) * 12);
+    memcpy(ms, ctx->ms, sizeof ctx->ms);
     if (launches) *launches = ctx->launches;
     return MCX_OK;
 }
