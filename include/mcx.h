@@ -193,7 +193,10 @@ int  mcx_timings_detail(mcx_ctx *ctx, float ms[4]);
 /* queue lengths of the last search (what the kernels between the stages worked on; the roofline figures of bench.py are
  * formed from them): [0] frames with a low-entropy window (k_seg), [1] records of the filter-pass queue, [2] of the
  * candidate queue, [3] of the seed queue ([1]-[3] include the few records a warp reserved and left empty), [4] ungapped
- * HSPs at or above the report floor; [5]-[7] reserved (0) */
+ * HSPs at or above the report floor; [5] gapped extensions the screening pass (k_gap_screen) handed to the complete DP
+ * (k_gap_dp), [6] extensions whose live window outgrew k_gap_dp's ring and went to the fallback (k_gap_dir); [7] reserved
+ * (0).  The environment variables MCX_GAP_SCREEN_ROWS (1..32), MCX_GAP_SCREEN_COLS (1..48) and MCX_GAP_DP_COLS (1..56)
+ * lower the limits at which these hand-offs happen (tests of the later paths; the results do not depend on them). */
 int  mcx_search_counters(mcx_ctx *ctx, int64_t out[8]);
 
 /* Measurement aid (SURVEY 8d): issue rate of the DPX instructions an affine-gap cell uses (viaddmax_s32 /

@@ -1460,14 +1460,18 @@ __global__ void k_gap_list(GapArgs A) {
 //    came as a nibble in global memory (what the binary keeps in its three trace matrices); k_gap_trace walks back from
 //    the best cell like the binary's CalRes and counts identities, columns, gap columns and gap runs.  (Carrying those
 //    statistics through the DP, as round 1 did, needs two more words per column: 768 bytes of shared memory per
-//    extension, 9 warps per SM, 32 % of the issue slots used.)  The live window [cs - 1, ce] never came near 56 columns
-//    in 25 M extensions (widest: 43) -- an extension that would is handed to the local-memory kernel k_gap_dir below,
-//    which stays as that fallback.
+//    extension, 9 warps per SM, 32 % of the issue slots used.)  An extension whose live window [cs - 1, ce] reaches 56
+//    columns is handed to the local-memory kernel k_gap_dir below, which stays as that fallback.  Measured on a B200
+//    (mcx_search_counters [5] / [6]): on 200,000 reads of the bench stream at 150 bp, 71,088 extensions went to
+//    k_gap_dp and none to k_gap_dir (widest window: 47 columns); on divergent homologs of the markers
+//    (tests/homologs.py) 15 of 2,325,109 at 150 bp (100,000 reads) and 9 of 523,564 at 500 bp (3,000 reads).
 // The first version of this stage (k_gap_dir for everything: rows of GROW ints in local memory, 6 LDL + 14 STL sites in
 // the score pass, 1.09 GB of DRAM writes per 226 M cells) ran at 110 GCUPS at 100 bp and 85 at 150 bp.
 #ifndef MCX_GAP_REFILL
 #define MCX_GAP_REFILL 24
 #endif
+// (the hand-off limits the kernels test are arguments: these sizes by default, lower with MCX_GAP_SCREEN_ROWS / _COLS and
+// MCX_GAP_DP_COLS, see gapped_stage)
 constexpr int SCR_COLS = 48;                   // columns of the screening pass (an extension that needs more goes to k_gap_dp)
 constexpr int RING = 64;                       // ring of k_gap_dp
 #ifndef MCX_SCR_NT
@@ -1525,7 +1529,8 @@ __device__ __forceinline__ ExtSetup ext_setup(const GapArgs &A, uint32_t item) {
 
 template <int NT>
 __global__ void __launch_bounds__(NT) k_gap_screen(GapArgs A, const unsigned long long *__restrict__ items,
-                                                   unsigned long long *__restrict__ gainers, unsigned long long *n_gainers) {
+                                                   unsigned long long *__restrict__ gainers, unsigned long long *n_gainers,
+                                                   int scr_rows, int scr_cols) {
     __shared__ __align__(16) int8_t s_bl[21 * 32];
     __shared__ uint32_t s_hf[SCR_COLS * NT];
     __shared__ uint32_t s_tq[(SCR_COLS / 4 + SCR_ROWS / 4) * NT];    // subject residues of columns 1 .. 48 and query residues of rows 1 .. 32, four per word
@@ -1602,7 +1607,7 @@ __global__ void __launch_bounds__(NT) k_gap_screen(GapArgs A, const unsigned lon
                     cells += j - 1;
                     if (!skip_tail) {                            // run on along the row by horizontal gaps
                         for (int jj = ce + 1; jj <= nD; ++jj) {
-                            if (jj >= SCR_COLS) { gain = true; busy = false; break; }   // needs more columns than this pass has: the full pass takes it
+                            if (jj >= scr_cols) { gain = true; busy = false; break; }   // needs more columns than this pass has: the full pass takes it
                             ++cells;
                             E = __viaddmax_s32(hl, -GIE, E - GE);
                             HF(jj) = pack_hf(E, E - GI);
@@ -1611,7 +1616,7 @@ __global__ void __launch_bounds__(NT) k_gap_screen(GapArgs A, const unsigned lon
                         }
                     }
                     if (!(1 < ce) || i >= nQ) busy = false;
-                    else if (i >= SCR_ROWS) { gain = true; busy = false; }   // more rows than this pass holds residues for
+                    else if (i >= scr_rows) { gain = true; busy = false; }   // more rows than this pass holds residues for
                     ++i;
                 }
             }
@@ -1640,7 +1645,8 @@ constexpr int DIR_ROW_WORDS = 1 + RING / 8;
 template <int NT>
 __global__ void __launch_bounds__(NT) k_gap_dp(GapArgs A, const unsigned long long *__restrict__ items, int64_t first, int64_t n_items,
                                                uint32_t *__restrict__ dirs, int rows_per_ext,
-                                               unsigned long long *__restrict__ wide, unsigned long long *n_wide, unsigned int *work) {
+                                               unsigned long long *__restrict__ wide, unsigned long long *n_wide, unsigned int *work,
+                                               int dp_cols) {
     __shared__ __align__(16) int8_t s_bl[21 * 32];
     __shared__ uint32_t s_ring[RING * NT];
     __shared__ uint32_t s_tr[(RING / 4) * NT];       // subject residues of the columns around the window, ring-indexed like the row
@@ -1693,7 +1699,7 @@ __global__ void __launch_bounds__(NT) k_gap_dp(GapArgs A, const unsigned long lo
             if (i <= nQ) {
                 // every column this row can touch must fit the ring next to column cs - 1 (8 columns to spare: a word of
                 // direction nibbles is written once per row)
-                if (min(ce, nD) - (cs - 1) >= RING - 8) over = true;
+                if (min(ce, nD) - (cs - 1) >= dp_cols) over = true;
                 else {
                     const int r0 = RI(cs - 1);
                     const uint32_t w0 = hf[r0];
@@ -1758,7 +1764,7 @@ __global__ void __launch_bounds__(NT) k_gap_dp(GapArgs A, const unsigned long lo
                     else if (cs <= jend) cells += jend - cs + 1;
                     if (!skip_tail) {
                         for (int jj = ce + 1; jj <= nD; ++jj) {          // run on along the row by horizontal gaps
-                            if (jj - (cs - 1) >= RING - 8) { over = true; break; }
+                            if (jj - (cs - 1) >= dp_cols) { over = true; break; }
                             ++cells;
                             const int a = hl - GIE, b = E - GE;
                             const uint32_t nib = (a > b ? 4u : 0u) | 8u | 1u;
@@ -3396,6 +3402,7 @@ struct SearchPlan {
 struct SearchTally {
     int64_t sampled = 0, examined = 0;
     unsigned long long segq = 0, pass = 0, cand = 0, seeds = 0, surv = 0;   // surv: ungapped HSPs of all chunks so far
+    unsigned long long gain = 0, wide = 0;                                   // extensions handed to k_gap_dp / to k_gap_dir
     float ms_qc = 0, ms_frames = 0, ms_seg = 0, ms_probe = 0, ms_kprobe = 0, ms_ext = 0, ms_kseed = 0, ms_gap = 0;
 };
 
@@ -3604,8 +3611,8 @@ static int seed_stage(mcx_ctx *ctx, const SearchPlan &S, int64_t nr_max, SearchT
 
 // gapped extension of the survivors [first, first + count): work list (padded with all-ones keys up to its bound, so that
 // it can be sorted without knowing its length on the host) -> sorted by remaining query length -> screening pass ->
-// complete DP + traceback for the extensions that gain -> (never seen: wide-window fallback) -> finish
-static int gapped_stage(mcx_ctx *ctx, const SearchPlan &S, int64_t first, int64_t count) {
+// complete DP + traceback for the extensions that gain -> (rare: wide-window fallback, see k_gap_dp) -> finish
+static int gapped_stage(mcx_ctx *ctx, const SearchPlan &S, int64_t first, int64_t count, SearchTally &T) {
     cudaStream_t st = ctx->stream;
     GapArgs G;
     G.L = ctx->par.read_length; G.fstride = S.fstride; G.db = ctx->db; G.frames = S.frames; G.surv = ctx->d_surv;
@@ -3631,10 +3638,19 @@ static int gapped_stage(mcx_ctx *ctx, const SearchPlan &S, int64_t first, int64_
     TRY(resident_blocks(ctx, k_gap_dir<GAP_NT, GW, false>, GAP_NT, 0, res_dir));
     TRY(resident_blocks(ctx, k_gap_dir<GAP_NT, GW, true>, GAP_NT, 0, res_dir2));
     auto grid = [](unsigned want, unsigned resident) { return std::max(1u, std::min(want, resident)); };
-    k_gap_screen<SNT><<<grid(((unsigned)(2 * G.n_surv) + SNT - 1) / SNT, res_screen), SNT, 0, st>>>(G, list1, gainers, ctx->d_cnt + C_ITEMS2);
+    // where the stage hands an extension on (screen -> k_gap_dp after this many rows or columns, k_gap_dp -> k_gap_dir once
+    // the live window spans this many columns): the sizes of the kernels' shared-memory rows by default; smaller values
+    // route work down the later paths (for tests: the results must not change)
+    int scr_rows = SCR_ROWS, scr_cols = SCR_COLS, dp_cols = RING - 8;
+    if (const char *e = getenv("MCX_GAP_SCREEN_ROWS")) scr_rows = std::min(SCR_ROWS, std::max(1, atoi(e)));
+    if (const char *e = getenv("MCX_GAP_SCREEN_COLS")) scr_cols = std::min(SCR_COLS, std::max(1, atoi(e)));
+    if (const char *e = getenv("MCX_GAP_DP_COLS")) dp_cols = std::min(RING - 8, std::max(1, atoi(e)));
+    k_gap_screen<SNT><<<grid(((unsigned)(2 * G.n_surv) + SNT - 1) / SNT, res_screen), SNT, 0, st>>>(G, list1, gainers, ctx->d_cnt + C_ITEMS2,
+                                                                                                   scr_rows, scr_cols);
     CK(cudaMemcpyAsync(ctx->h_cnt + C_ITEMS2, ctx->d_cnt + C_ITEMS2, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
     TRY(sync_stream(ctx));
     const int64_t n_gain = (int64_t)ctx->h_cnt[C_ITEMS2];
+    T.gain += (unsigned long long)n_gain;
     // complete DP + traceback of the extensions that gain, in batches that bound the direction scratch
     const int rows_per_ext = S.maxm;
     const int64_t per_ext = (int64_t)rows_per_ext * DIR_ROW_WORDS;
@@ -3646,15 +3662,18 @@ static int gapped_stage(mcx_ctx *ctx, const SearchPlan &S, int64_t first, int64_
         const int64_t ng = std::min(batch, n_gain - g0);
         CK(cudaMemsetAsync(ctx->d_cnt + C_WORK1, 0, sizeof(unsigned long long), st));
         k_gap_dp<FNT><<<grid((unsigned)((ng + FNT - 1) / FNT), res_dp), FNT, 0, st>>>(
-            G, gainers, g0, ng, ctx->d_dirs, rows_per_ext, wide, ctx->d_cnt + C_NWIDE, reinterpret_cast<unsigned int *>(ctx->d_cnt + C_WORK1));
+            G, gainers, g0, ng, ctx->d_dirs, rows_per_ext, wide, ctx->d_cnt + C_NWIDE, reinterpret_cast<unsigned int *>(ctx->d_cnt + C_WORK1), dp_cols);
         k_gap_trace<<<(unsigned)((ng + 127) / 128), 128, 0, st>>>(G, gainers, g0, ng, ctx->d_dirs, rows_per_ext);
         ctx->launches += 2;
     }
-    // fallback for extensions whose window outgrew the ring: score pass + statistics pass with rows in local memory
-    unsigned long long *wide2 = ctx->d_gitems + G.n_surv;
+    // fallback for extensions whose window outgrew the ring: score pass + statistics pass with rows in local memory.  The
+    // list of the statistics pass takes the place of the sorted work list (read by the screen only): `wide` can hold up to
+    // all 2 n_surv extensions, so no part of [0, 2 n_surv) is free while the score pass reads it.
+    unsigned long long *wide2 = list1;
     unsigned int *work2 = reinterpret_cast<unsigned int *>(ctx->d_cnt + C_WORK2), *work3 = reinterpret_cast<unsigned int *>(ctx->d_cnt + C_NWIDE + 2);
     k_gap_dir<GAP_NT, GW, false><<<grid(64, res_dir), GAP_NT, 0, st>>>(G, wide, ctx->d_cnt + C_NWIDE, wide2, ctx->d_cnt + C_NWIDE + 1, work2);
     k_gap_dir<GAP_NT, GW, true><<<grid(64, res_dir2), GAP_NT, 0, st>>>(G, wide2, ctx->d_cnt + C_NWIDE + 1, nullptr, nullptr, work3);
+    CK(cudaMemcpyAsync(ctx->h_cnt + C_NWIDE, ctx->d_cnt + C_NWIDE, sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));   // read after the chunk's sync
     ctx->launches += 8;
     k_gap_finish<<<(unsigned)((G.n_surv + 255) / 256), 256, 0, st>>>(G);
     ctx->launches += 3;
@@ -3680,6 +3699,7 @@ static int classify_and_collect(mcx_ctx *ctx, const SearchTally &T, bool stored)
     R.n_seed_hits = (int64_t)T.surv;
     ctx->work[0] = (int64_t)T.segq; ctx->work[1] = (int64_t)T.pass; ctx->work[2] = (int64_t)T.cand;
     ctx->work[3] = (int64_t)T.seeds; ctx->work[4] = (int64_t)T.surv;
+    ctx->work[5] = (int64_t)T.gain; ctx->work[6] = (int64_t)T.wide;
     const int64_t ns = (int64_t)T.surv;
     CK(cudaEventRecord(ctx->ev[EV_SORT0], st));
     if (ns > 0) {
@@ -3765,9 +3785,11 @@ extern "C" int mcx_search(mcx_ctx *ctx, int64_t quota) {
         const unsigned long long surv_before = T.surv;
         TRY(seed_stage(ctx, S, nr_max, T));
         T.sampled += nr < 0 ? (int64_t)ctx->h_cnt[C_NKEPT] : nr;
-        if (T.surv > surv_before) TRY(gapped_stage(ctx, S, (int64_t)surv_before, (int64_t)(T.surv - surv_before)));
+        const bool gapped = T.surv > surv_before;
+        if (gapped) TRY(gapped_stage(ctx, S, (int64_t)surv_before, (int64_t)(T.surv - surv_before), T));
         CK(cudaEventRecord(ctx->ev[EV_GAP1], st));
         TRY(sync_stream(ctx));
+        if (gapped) T.wide += ctx->h_cnt[C_NWIDE];
         T.ms_qc += elapsed_ms(ctx->ev[EV_QC0], ctx->ev[EV_FRAMES0]);
         T.ms_frames += elapsed_ms(ctx->ev[EV_FRAMES0], ctx->ev[EV_SEG0]);
         T.ms_seg += elapsed_ms(ctx->ev[EV_SEG0], ctx->ev[EV_PROBE0]);

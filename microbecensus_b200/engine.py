@@ -366,7 +366,8 @@ class MarkerSearch:
         """queue lengths of the last search (include/mcx.h mcx_search_counters)"""
         out = (C.c_int64 * 8)()
         self._ck(self.lib.mcx_search_counters(self.ctx, C.byref(out)))
-        return dict(zip(("seg_frames", "filter_passes", "candidates", "seeds", "ungapped_hsps"), (int(x) for x in out[:5])))
+        return dict(zip(("seg_frames", "filter_passes", "candidates", "seeds", "ungapped_hsps", "gap_dp_extensions",
+                         "gap_wide_extensions"), (int(x) for x in out[:7])))
 
     def timings(self):
         ms = (C.c_float * 12)()
